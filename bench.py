@@ -1,6 +1,6 @@
 """bench.py — the headline benchmark of the raybuffer path (BASELINE.json: frames/sec on mill 1024^3 at 1080p & 4K).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 1..5] [--mode views|rays] [--res WxH]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 1..5] [--mode views|rays] [--res WxH] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workloads (config.workload; BASELINE.json `configs`, made concrete in SURVEY.md §8(d)):
@@ -50,11 +50,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree it runs from may be read-only: bench.py leaves nothing in it
 
 MILL = os.path.join(ROOT, "tests", "data", "mill.obj")
 FRAMES_PER_STEP = 60
 METRIC = "frames/sec @4K, mill 1024^3, BenchmarkPath 60 poses"
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 48 << 20
 
 
 def parse_args():
@@ -76,11 +78,19 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-1080p", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip at_inflight, d2h_ceiling and rays_sharded (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the frames of the last step to DIR/frames.npy (views mode, rank 0): float64 pixel "
+                         "values (the packed 32-bit colours, exact) of every view at a fixed seeded sample of pixel positions, "
+                         f"at most {DUMP_BYTES >> 20} MiB; the inputs are the same from run to run, so two builds compare output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.res is None:
         a.res = {1: "3840x2160", 2: "1920x1080", 3: "3840x2160", 4: "7680x4320", 5: "1280x720"}[a.config]
     if a.mode == "auto":
         a.mode = "rays" if a.config == 4 else "views"
+    if a.dump_outputs and (a.mode != "views" or a.impl != "b200"):
+        ap.error("--dump-outputs writes the frames of the GPU views path (--impl b200, --mode views)")
     return a
 
 
@@ -280,6 +290,26 @@ class CpuPath:
         what = ("reference C# translated to C++ (oracle/_ref: cs2cpp.py, g++ -O2 -ffp-contract=off; not .NET, not Burst)" if self.kind == "reference"
                 else "hand C++ restatement (oracle/cpuvox_oracle.cpp)")
         return f"Phase 1 = {what}, Phase 2 = per-pixel restatement of the blit shader; {self.threads} host threads"
+
+
+def dump_frames(directory, cv, N, rm, setups, W, H):
+    """--dump-outputs, right after the timed steps: every view's frame of the step, as cvx_draw_batch hands them to a caller.
+    The device-only timed steps keep only the last view's frame readable, so the same batch is drawn once more into host memory;
+    its last frame must equal the one the timed steps left behind. A 4K step is 2 GB of frames: a seeded sample of pixel
+    positions (the same for every view) is written as float64, which holds the 32-bit colours exactly."""
+    last = rm.read_frame()
+    frames = cv.alloc_pinned((len(setups), H, W))
+    try:
+        rm.draw_batch(setups, frames)
+        if not np.array_equal(frames[-1], last):
+            raise SystemExit("--dump-outputs: drawing the step again gave a different last frame")
+        per_view = min(W * H, DUMP_BYTES // (8 * len(setups)))
+        idx = np.sort(np.random.default_rng(0).choice(W * H, per_view, replace=False))
+        out = frames.reshape(len(setups), -1)[:, idx].astype(np.float64)
+    finally:
+        N.lib.cvx_free_pinned(frames.ctypes.data)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "frames.npy"), out)
 
 
 def config_block(a, name, W, H, frames_per_step, extra=None):
@@ -585,6 +615,8 @@ def run_b200(a, rank, local_rank, world_size):
         ms, p1, p2, n, launches, span = time_path(torch, dist, rm, setups, steps, a.warmup, device, flush, world_size)
         if sampler:
             clocks = sampler.stop(*span)
+        if ri == 0 and rank == 0 and a.dump_outputs:
+            dump_frames(a.dump_outputs, cv, N, rm, setups, w, h)
         # the same launches one view at a time: exclusive kernel durations (outside the timed region, reported beside it)
         rm.set_frames_in_flight(1)
         _, x1, x2, xn, _, _ = time_path(torch, dist, rm, setups, 1, 1, device, flush, world_size)
