@@ -6,6 +6,8 @@ shared library has not been built — there is no CPU or Python fallback.
 """
 from .native import LIB_PATH, CvxError, FrameSetup, LOD_LEVELS  # noqa: F401
 from .host import (  # noqa: F401
+    RAY_DTYPE,
+    RAY_HIT_DTYPE,
     SKYBOX_ARGB,
     CameraPose,
     RenderManager,
@@ -16,6 +18,8 @@ from .host import (  # noqa: F401
     benchmark_path,
     benchmark_pose,
     frame_setup,
+    make_rays,
+    screen_ray,
     setup_lods,
     write_bmp,
 )

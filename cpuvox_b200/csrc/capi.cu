@@ -19,11 +19,14 @@
 #include "host_frame.h"
 #include "jpeg_encoder.h"
 #include "nvtx_ranges.h"
+#include "raycast.h"
 #include "world_builder.h"
 
 static_assert(sizeof(cvx_ray_state) == sizeof(cvxd_ray_state), "ray state layout");
 static_assert(sizeof(cvx_counters) == sizeof(cvxd_counters), "counter layout");
 static_assert(CVX_LOD_LEVELS == CVXD_LODS, "lod levels");
+static_assert(sizeof(cvx_ray) == sizeof(cvxd_ray) && sizeof(cvx_ray) == 32, "ray layout");
+static_assert(sizeof(cvx_ray_hit) == sizeof(cvxd_ray_hit) && sizeof(cvx_ray_hit) == 32, "ray hit layout");
 
 #define CVX_MAX_SLOTS 16
 #define CVX_DEFAULT_SLOTS 6
@@ -90,6 +93,8 @@ struct cvx_ctx {
     size_t ringFrameBytes = 0;
     int groupSize = 0;                  // lanes per ray in phase 1: 0 = auto, 8, 16, 32
     int generalPath = 0;                // 1 = never use the boundary-table kernel
+    void* rayScratch = nullptr;         // cvx_raycast with host arrays: rays then hits, grown to the largest call
+    size_t rayScratchBytes = 0;
     std::string error;
 };
 
@@ -288,6 +293,12 @@ void free_world(cvx_ctx* ctx) {
     memset(&ctx->world, 0, sizeof ctx->world);
 }
 
+void free_ray_scratch(cvx_ctx* ctx) {
+    cudaFree(ctx->rayScratch);
+    ctx->rayScratch = nullptr;
+    ctx->rayScratchBytes = 0;
+}
+
 // Takes ownership of `dblob` (a whole LOD blob in device memory: column_count 12-byte headers + element area), builds the Phase-1
 // tables from it on the device (world_builder_gpu.cu: the same tables world_transcode.h builds on the host for the emulator; it
 // also validates what the kernels index with) and makes it LOD `lod` of the context's world.
@@ -369,6 +380,7 @@ int cvx_destroy(cvx_ctx* ctx) {
     cvx_ring_close(ctx);
     free_resolution(ctx);
     free_world(ctx);
+    free_ray_scratch(ctx);
     for (cudaEvent_t e : ctx->profEvents) cudaEventDestroy(e);
     cvxjpeg::destroy(ctx->jpeg);
     cudaFree(ctx->counters);
@@ -432,6 +444,7 @@ int cvx_world_free(cvx_ctx* ctx) {
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     free_world(ctx);
+    free_ray_scratch(ctx);
     return CVX_OK;
 }
 
@@ -829,6 +842,41 @@ int cvx_world_build_from_mesh(cvx_ctx* ctx, const float* positions, const uint8_
     if (r) { free_world(ctx); return ctx->error.empty() || r != CVX_ERR_FORMAT ? fail(ctx, r, "device world build failed: %s", err.c_str()) : r; }
     if (out_dims) { out_dims[0] = dims[0]; out_dims[1] = dims[1]; out_dims[2] = dims[2]; }
     if (out_voxel_counts) for (int i = 0; i < CVX_LOD_LEVELS; i++) out_voxel_counts[i] = i < n_lods ? b.lods[i].voxelCount : 0;
+    return CVX_OK;
+}
+
+// Ray queries (raycast.h, raycast_kernels.cu): the kernel reads the world tables the context holds at the time of the call, on the
+// context's stream, so it follows any draw or batch join queued there and a later world replacement (which synchronises that stream
+// before freeing the old tables) cannot pull them from under it.
+int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device) {
+    if (!ctx) return CVX_ERR_INVALID_ARGUMENT;
+    if (ctx->world.lod_count <= 0) return fail(ctx, CVX_ERR_NO_WORLD, "no world uploaded");
+    if (lod < 0 || lod >= CVX_LOD_LEVELS || !ctx->world.lods[lod].headers) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "LOD %d is not uploaded", lod);
+    if (n < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "n = %d < 0", n);
+    if (n > 0 && (!rays || !out)) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "rays or hits is NULL");
+    if (n == 0) return CVX_OK;
+    CU(ctx, cudaSetDevice(ctx->device));
+    const bool bounds = ctx->lodRegular[lod] && !ctx->generalPath;
+    if (on_device) {
+        CU(ctx, cvxd_launch_raycast(ctx->world, lod, (const cvxd_ray*)rays, (cvxd_ray_hit*)out, n, bounds, ctx->stream));
+        ctx->launches++;
+        return CVX_OK;
+    }
+    const size_t rayBytes = (size_t)n * sizeof(cvx_ray), need = rayBytes + (size_t)n * sizeof(cvx_ray_hit);
+    if (need > ctx->rayScratchBytes) {
+        CU(ctx, cudaStreamSynchronize(ctx->stream));
+        free_ray_scratch(ctx);
+        cudaError_t e = cudaMalloc(&ctx->rayScratch, need);
+        if (e != cudaSuccess) { ctx->rayScratch = nullptr; return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "ray scratch allocation failed: %s", cudaGetErrorString(e)); }
+        ctx->rayScratchBytes = need;
+    }
+    cvxd_ray* dRays = (cvxd_ray*)ctx->rayScratch;
+    cvxd_ray_hit* dHits = (cvxd_ray_hit*)((uint8_t*)ctx->rayScratch + rayBytes);
+    CU(ctx, cudaMemcpyAsync(dRays, rays, rayBytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cvxd_launch_raycast(ctx->world, lod, dRays, dHits, n, bounds, ctx->stream));
+    ctx->launches++;
+    CU(ctx, cudaMemcpyAsync(out, dHits, (size_t)n * sizeof(cvx_ray_hit), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
     return CVX_OK;
 }
 

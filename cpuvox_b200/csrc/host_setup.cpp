@@ -235,6 +235,11 @@ struct SegmentSolver {
     }
 };
 
+// ScreenPointToRay in camera space (A8): the point of pixel (px, py) on the plane z = 1, i.e. the unnormalised direction
+Vec3 camera_ray(float px, float py, int W, int H, float aspect, float tanHalf) {
+    return Vec3{(2.0f * px / W - 1.0f) * aspect * tanHalf, (2.0f * py / H - 1.0f) * tanHalf, 1.0f};
+}
+
 struct CurveKey { float time; float value[3]; float inSlope[3]; float outSlope[3]; };
 
 // Non-weighted AnimationCurve segment: cubic Hermite (A9)
@@ -303,9 +308,7 @@ void cvx_host_setup_lods(int32_t world_max_dimension, int32_t res_x, int32_t res
     const int midW = res_x / 2, midH = res_y / 2;
     const float tanHalf = (float)tan((double)(fov_y_degrees * kDeg2Rad * 0.5f));
     const float aspect = (float)res_x / (float)res_y;
-    auto ray_dir = [&](float px, float py) { // ScreenPointToRay direction in camera space (A8)
-        return unit(Vec3{(2.0f * px / res_x - 1.0f) * aspect * tanHalf, (2.0f * py / res_y - 1.0f) * tanHalf, 1.0f});
-    };
+    auto ray_dir = [&](float px, float py) { return unit(camera_ray(px, py, res_x, res_y, aspect, tanHalf)); };
     const Vec3 a = ray_dir((float)midW, (float)midH), b = ray_dir(midW + pixelW, midH + pixelH);
     bool found[CVX_LOD_LEVELS] = {false};
     float at[CVX_LOD_LEVELS] = {0};
@@ -320,6 +323,17 @@ void cvx_host_setup_lods(int32_t world_max_dimension, int32_t res_x, int32_t res
     }
     found[CVX_LOD_LEVELS - 1] = true; at[CVX_LOD_LEVELS - 1] = 2.0f; // last LOD never ends
     for (int i = 0; i < CVX_LOD_LEVELS; i++) out_lod_distances[i] = ceilf((found[i] ? at[i] : 2.0f) * clipMax);
+}
+
+void cvx_host_screen_ray(const cvx_pose* pose, float px, float py, float out_origin[3], float out_direction[3]) {
+    const float tanHalf = (float)tan((double)(pose->fov_y_degrees * kDeg2Rad * 0.5f));
+    const float aspect = (float)pose->pixel_width / (float)pose->pixel_height;
+    const Quat rot = {pose->rotation[0], pose->rotation[1], pose->rotation[2], pose->rotation[3]};
+    const Vec3 cam = camera_ray(px, py, pose->pixel_width, pose->pixel_height, aspect, tanHalf);
+    const Vec3 onNear = rotate(rot, Vec3{cam.x * pose->near_clip, cam.y * pose->near_clip, pose->near_clip});
+    const Vec3 dir = rotate(rot, unit(cam));
+    out_origin[0] = pose->position[0] + onNear.x; out_origin[1] = pose->position[1] + onNear.y; out_origin[2] = pose->position[2] + onNear.z;
+    out_direction[0] = dir.x; out_direction[1] = dir.y; out_direction[2] = dir.z;
 }
 
 int cvx_host_frame_setup(const cvx_pose* pose, const float lod_distances[CVX_LOD_LEVELS], int32_t world_dim_y, cvx_frame_setup* out) {

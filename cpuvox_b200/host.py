@@ -171,6 +171,33 @@ def frame_setup(pose: CameraPose, width: int, height: int, lod_distances: np.nda
     return out
 
 
+# cvx_ray / cvx_ray_hit as numpy records (include/cpuvox_b200.h)
+RAY_DTYPE = np.dtype([("origin", "<f4", 3), ("max_distance", "<f4"), ("direction", "<f4", 3), ("reserved", "<i4")])
+RAY_HIT_DTYPE = np.dtype([("hit", "<i4"), ("face", "<i4"), ("cell", "<i4", 3), ("distance", "<f4"), ("color", "<u4"), ("steps", "<i4")])
+
+
+def make_rays(origins, directions, max_distance=np.inf) -> np.ndarray:
+    """Pack origins (n, 3), directions (n, 3) and max_distance (scalar or (n,)) into a cvx_ray array."""
+    origins = np.asarray(origins, dtype=np.float32).reshape(-1, 3)
+    directions = np.asarray(directions, dtype=np.float32).reshape(-1, 3)
+    if origins.shape != directions.shape:
+        raise ValueError(f"origins {origins.shape} and directions {directions.shape} differ")
+    rays = np.zeros(origins.shape[0], dtype=RAY_DTYPE)
+    rays["origin"] = origins
+    rays["direction"] = directions
+    rays["max_distance"] = max_distance
+    return rays
+
+
+def screen_ray(pose: CameraPose, px: float, py: float, width: int, height: int) -> Tuple[np.ndarray, np.ndarray]:
+    """Camera.ScreenPointToRay (cvx_host_screen_ray): pixel (px, py) in Unity screen space (bottom-left origin) of a width x height
+    camera; returns (origin on the near plane, normalised direction), float32 (3,) each."""
+    p = pose.to_native(width, height)
+    o, d = (C.c_float * 3)(), (C.c_float * 3)()
+    lib.cvx_host_screen_ray(C.byref(p), px, py, C.byref(o), C.byref(d))
+    return np.array(o[:], dtype=np.float32), np.array(d[:], dtype=np.float32)
+
+
 class RenderManager:
     """RenderManager (Assets/Code/RenderManager.cs) with its Phase-1 jobs and Phase-2 blit on the GPU."""
 
@@ -319,6 +346,29 @@ class RenderManager:
 
     def sync(self):
         self._ck(lib.cvx_sync(self._ctx))
+
+    # -- ray queries (cvx_raycast) --------------------------------------------------------------------
+    def raycast_rays(self, rays: np.ndarray, lod: int = 0) -> np.ndarray:
+        """cvx_raycast over a RAY_DTYPE array (host path): returns the RAY_HIT_DTYPE hits."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        hits = np.zeros(rays.shape[0], dtype=RAY_HIT_DTYPE)
+        self._ck(lib.cvx_raycast(self._ctx, _ptr(rays), rays.shape[0], lod, _ptr(hits), 0))
+        return hits
+
+    def raycast(self, origins, directions, max_distance=np.inf, lod: int = 0) -> np.ndarray:
+        """First voxel each ray hits at LOD `lod`: origins / directions (n, 3) in world units (directions need not be normalised),
+        max_distance a scalar or (n,). Returns a RAY_HIT_DTYPE array (hit 1 / 0 / -1 invalid, face, cell, distance, color, steps)."""
+        return self.raycast_rays(make_rays(origins, directions, max_distance), lod)
+
+    def raycast_device(self, rays_ptr: int, hits_ptr: int, n: int, lod: int = 0):
+        """cvx_raycast on device arrays (n cvx_ray in, n cvx_ray_hit out; e.g. torch tensors' data_ptr()), ordered on the context's
+        stream; returns at once."""
+        self._ck(lib.cvx_raycast(self._ctx, C.c_void_p(rays_ptr), n, lod, C.c_void_p(hits_ptr), 1))
+
+    def pick(self, pose: CameraPose, px: float, py: float, lod: int = 0, max_distance: float = np.inf) -> np.void:
+        """The voxel under screen pixel (px, py) (bottom-left origin) of `pose` at this context's resolution: one RAY_HIT_DTYPE record."""
+        o, d = screen_ray(pose, px, py, self.width, self.height)
+        return self.raycast(o, d, max_distance, lod)[0]
 
     # -- outputs ----------------------------------------------------------------------------------
     def read_frame(self, out: Optional[np.ndarray] = None) -> np.ndarray:

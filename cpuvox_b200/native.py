@@ -104,6 +104,26 @@ class RayState(C.Structure):
     ]
 
 
+class Ray(C.Structure):  # cvx_ray: a ray query (no reference analogue), 32 bytes
+    _fields_ = [
+        ("origin", C.c_float * 3),
+        ("max_distance", C.c_float),
+        ("direction", C.c_float * 3),
+        ("reserved", C.c_int32),
+    ]
+
+
+class RayHit(C.Structure):  # cvx_ray_hit, 32 bytes
+    _fields_ = [
+        ("hit", C.c_int32),
+        ("face", C.c_int32),
+        ("cell", C.c_int32 * 3),
+        ("distance", C.c_float),
+        ("color", C.c_uint32),
+        ("steps", C.c_int32),
+    ]
+
+
 # every symbol include/cpuvox_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U32, _F = C.c_int32, C.c_int64, C.c_uint32, C.c_float
@@ -152,11 +172,13 @@ SYMBOLS = {
     "cvx_draw_sharded": (C.c_int, [_P, C.POINTER(FrameSetup), C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
     "cvx_ring_consume": (C.c_int, [_P, C.c_int64, _P, C.POINTER(_P)]),
     "cvx_ring_status": (C.c_int, [_P]),
+    "cvx_raycast": (C.c_int, [_P, _P, _I32, _I32, _P, _I32]),
     "cvx_debug_ray_setup": (C.c_int, [_P, C.POINTER(FrameSetup), C.POINTER(RayState), _I32]),
     "cvx_debug_ray_timing": (C.c_int, [_P, C.POINTER(FrameSetup), _P, _I32]),
     "cvx_host_quat_euler": (None, [_F, _F, _F, C.POINTER(_F * 4)]),
     "cvx_host_limit_rotation_horizon": (None, [C.POINTER(Pose)]),
     "cvx_host_setup_lods": (None, [_I32, _I32, _I32, _F, _F, C.POINTER(_F * LOD_LEVELS)]),
+    "cvx_host_screen_ray": (None, [C.POINTER(Pose), _F, _F, C.POINTER(_F * 3), C.POINTER(_F * 3)]),
     "cvx_host_frame_setup": (C.c_int, [C.POINTER(Pose), C.POINTER(_F * LOD_LEVELS), _I32, C.POINTER(FrameSetup)]),
     "cvx_host_benchmark_pose": (None, [_F, C.POINTER(_I32 * 3), C.POINTER(Pose)]),
     "cvx_host_benchmark_length": (_F, []),

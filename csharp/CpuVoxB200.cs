@@ -49,6 +49,26 @@ public static unsafe class CpuVoxB200
 	[StructLayout(LayoutKind.Sequential)]
 	public struct Config { public int Device; public int Flags; }
 
+	// Ray queries against the resident world (cvx_raycast; no reference analogue). 32 bytes each.
+	[StructLayout(LayoutKind.Sequential)]
+	public struct Ray
+	{
+		public float OriginX, OriginY, OriginZ;
+		public float MaxDistance; // float.PositiveInfinity = unbounded
+		public float DirectionX, DirectionY, DirectionZ; // need not be normalised
+		public int Reserved;
+	}
+
+	[StructLayout(LayoutKind.Sequential)]
+	public struct RayHit
+	{
+		public int Hit;  // 1 hit, 0 miss, -1 invalid ray
+		public int Face; // entry face: 0 -X, 1 +X, 2 -Y, 3 +Y, 4 -Z, 5 +Z; 6 = origin inside the voxel
+		public int CellX, CellY, CellZ; // LOD cell
+		public float Distance; // world units along the normalised direction
+		public uint Color; // ColorARGB32
+		public int Steps;
+	}
 	[DllImport(LIB)] public static extern int cvx_create(ref Config config, out IntPtr ctx);
 	[DllImport(LIB)] public static extern int cvx_destroy(IntPtr ctx);
 	[DllImport(LIB)] public static extern IntPtr cvx_last_error(IntPtr ctx);
@@ -66,6 +86,8 @@ public static unsafe class CpuVoxB200
 	[DllImport(LIB)] public static extern int cvx_device_frame(IntPtr ctx, out IntPtr devicePtr, out long bytes);
 	[DllImport(LIB)] public static extern int cvx_clear_raybuffers(IntPtr ctx, uint argb);
 	[DllImport(LIB)] public static extern int cvx_set_option(IntPtr ctx, int option, int value); // 1 lanes per ray, 2 counters, 3 general path, 4 views in flight
+	// onDevice 0: host arrays, returns with the hits; onDevice 1: device pointers, ordered on the context's stream
+	[DllImport(LIB)] public static extern int cvx_raycast(IntPtr ctx, Ray* rays, int n, int lod, RayHit* hits, int onDevice);
 	// world production on the GPU (VoxelizerHelper + WorldBuilder.ToFinalColumn + World.DownSample as CUDA kernels); positions = n x float3
 	// already in mesh space, colors32 = n x Color32; flips = int[3]. The first returns a builder handle (read its LOD blobs with
 	// cvx_builder_lod, free with cvx_builder_free), the second installs the result as the context's world without a host copy.

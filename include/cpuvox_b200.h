@@ -234,6 +234,37 @@ int cvx_draw_sharded(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_beg
 int cvx_ring_consume(cvx_ctx* ctx, int64_t view_index, void* dst_host, void** out_device_frame);
 int cvx_ring_status(cvx_ctx* ctx);
 
+/* ---- ray queries against the resident world (no reference analogue: SURVEY.md lists no ray query in the reference) -----------
+ * Picking, hit-scan, line of sight and depth probes: what does a ray hit first? The query runs at one uploaded LOD j (cells of
+ * 2^j world units); the ray starts at `origin` (world units), `direction` need not be normalised, and `distance` is measured along
+ * the normalised direction in world units, up to `max_distance` (+inf allowed). The exact definition, which the device kernel
+ * follows bit for bit in IEEE fp32, is DESIGN.md §3.5.
+ *   hit       1 = hit, 0 = miss, -1 = invalid ray (zero-length direction, or a NaN / infinite input other than max_distance = +inf)
+ *   face      outward normal of the face the ray entered the hit cell through: 0 -X, 1 +X, 2 -Y, 3 +Y, 4 -Z, 5 +Z;
+ *             6 = the origin lies inside the solid cell (distance 0)
+ *   cell      the hit cell in LOD-j cells; color its ColorARGB32; steps = cells the definition tests (also on a miss)
+ * A miss or an invalid ray has every field but `steps` zero. */
+typedef struct cvx_ray {
+    float origin[3];
+    float max_distance;
+    float direction[3];
+    int32_t reserved;
+} cvx_ray; /* 32 bytes */
+typedef struct cvx_ray_hit {
+    int32_t hit;
+    int32_t face;
+    int32_t cell[3];
+    float distance;
+    uint32_t color;
+    int32_t steps;
+} cvx_ray_hit; /* 32 bytes */
+/* on_device == 0: rays / out are host arrays; the call returns when the hits are in `out` (device scratch grows to the largest n
+ * and is freed by cvx_world_free / cvx_destroy). on_device != 0: device pointers; the query is ordered on the context's stream
+ * after whatever is queued there and the call returns at once. Either way it reads the world uploaded at the time of the call.
+ * CVX_ERR_NO_WORLD without a world; CVX_ERR_INVALID_ARGUMENT for a LOD that is not uploaded, n < 0, or NULL arrays with n > 0;
+ * n == 0 does nothing. CVX_OPT_GENERAL_PATH 1 makes it read runs from the element area (same results). */
+int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device);
+
 /* Debug: dump the per-ray state after RaySetupJob/DDASetupJob/TraceToFirstColumnJob
  * (DrawSegmentRayJob.cs:12-144) for every flat ray index; 18 x 4 bytes per ray, see cvx_ray_state. */
 typedef struct cvx_ray_state {
@@ -286,6 +317,9 @@ void cvx_host_setup_lods(int32_t world_max_dimension, int32_t res_x, int32_t res
  * GetGenericSegmentParameters x4 (:402-501), CameraData ctor (CameraData.cs:18-36). */
 int cvx_host_frame_setup(const cvx_pose* pose, const float lod_distances[CVX_LOD_LEVELS],
                          int32_t world_dim_y, cvx_frame_setup* out);
+/* Camera.ScreenPointToRay for pixel (px, py) in Unity screen space (bottom-left origin, the framebuffer's rows) of a camera of
+ * pose->pixel_width x pose->pixel_height: the origin on the near plane, the direction normalised (feed it to cvx_raycast). */
+void cvx_host_screen_ray(const cvx_pose* pose, float px, float py, float out_origin[3], float out_direction[3]);
 /* RenderManager.DrawWorld for a batch of cameras on a host without UnityEngine (RenderManager.cs:111-194; with limit_rotation_horizon != 0
  * also UnityManager.LimitRotationHorizon, UnityManager.cs:181): the library computes each view's frame setup from its pose at the
  * context's resolution (pixel_width / pixel_height of the poses are ignored) and renders the views like cvx_draw_batch. */

@@ -14,6 +14,7 @@ unsigned long long* emu_stats = nullptr;
 #include "../../cpuvox_b200/csrc/raybuffer_kernels.cu"
 #include "../../cpuvox_b200/csrc/host_frame.h"
 #include "../../cpuvox_b200/csrc/world_transcode.h"
+#include "../../cpuvox_b200/csrc/raycast.h"
 
 struct emu_world {
     cvxh_lod_tables tables[CVXD_LODS];
@@ -115,6 +116,27 @@ int emu_phase1(const emu_world* w, const cvx_frame_setup* setup, int W, int H, u
     worker();
     for (auto& t : pool) t.join();
     return n;
+}
+
+// cvx_raycast's traversal (raycast.h) for rays [0, n) at LOD lod: one call per ray, as one device thread runs it. general != 0 reads
+// runs from the element area even for a regular LOD (CVX_OPT_GENERAL_PATH).
+int emu_raycast(const emu_world* w, int lod, const cvxd_ray* rays, int n, cvxd_ray_hit* hits, int general, int threads) {
+    if (lod < 0 || lod >= w->w.lod_count || n < 0) return -1;
+    const bool bounds = w->tables[lod].regular && !general;
+    std::atomic<int> next{0};
+    if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
+    auto worker = [&]() {
+        for (;;) {
+            const int b = next.fetch_add(1024);
+            if (b >= n) break;
+            for (int i = b; i < n && i < b + 1024; i++) cvxr_cast(w->w, lod, rays[i], bounds, hits[i]);
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 1; t < threads; t++) pool.emplace_back(worker);
+    worker();
+    for (auto& t : pool) t.join();
+    return 0;
 }
 
 } // extern "C"
