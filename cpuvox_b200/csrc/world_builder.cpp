@@ -151,8 +151,8 @@ void assemble_blob(Blob& blob, int columnCount, int64_t slots, const std::vector
 }
 
 
-inline uint8_t to_byte(float c) { // Color -> Color32: round(clamp01(c)*255), half-to-even (SURVEY A10)
-    float v = c < 0.0f ? 0.0f : (c > 1.0f ? 1.0f : c);
+inline uint8_t to_byte(float c) { // Color -> Color32: round(clamp01(c)*255), half-to-even (SURVEY A10); NaN -> 0
+    float v = c > 0.0f ? (c < 1.0f ? c : 1.0f) : 0.0f;
     return (uint8_t)rintf(v * 255.0f);
 }
 inline int next_pow2(int n) { int p = 1; while (p < n) p <<= 1; return n <= 0 ? 0 : p; } // Mathf.NextPowerOfTwo (A11)
@@ -179,8 +179,10 @@ void voxelize_triangle(const V3 pa, const V3 pb, const V3 pc, const uint8_t* c0,
     a = a + normalize(a - mid) * 0.5f;
     b = b + normalize(b - mid) * 0.5f;
     c = c + normalize(c - mid) * 0.5f;
-    V3 mn = {std::min(a.x, std::min(b.x, c.x)), std::min(a.y, std::min(b.y, c.y)), std::min(a.z, std::min(b.z, c.z))};
-    V3 mx = {std::max(a.x, std::max(b.x, c.x)), std::max(a.y, std::max(b.y, c.y)), std::max(a.z, std::max(b.z, c.z))};
+    // math.min / math.max ignore a NaN operand, as fminf / fmaxf do: a corner on the centroid (normalize(0) = NaN) drops out of
+    // the box, which then spans the other two corners (DESIGN.md §3.4)
+    V3 mn = {fminf(a.x, fminf(b.x, c.x)), fminf(a.y, fminf(b.y, c.y)), fminf(a.z, fminf(b.z, c.z))};
+    V3 mx = {fmaxf(a.x, fmaxf(b.x, c.x)), fmaxf(a.y, fmaxf(b.y, c.y)), fmaxf(a.z, fmaxf(b.z, c.z))};
     int lo[3] = {clampi(f2i(floorf(mn.x)), 0, maxDim[0]), clampi(f2i(floorf(mn.y)), 0, maxDim[1]), clampi(f2i(floorf(mn.z)), 0, maxDim[2])};
     int hi[3] = {clampi(f2i(ceilf(mx.x)), 0, maxDim[0]), clampi(f2i(ceilf(mx.y)), 0, maxDim[1]), clampi(f2i(ceilf(mx.z)), 0, maxDim[2])};
     float col0[3] = {c0[0] / 255.0f, c0[1] / 255.0f, c0[2] / 255.0f};
@@ -348,9 +350,12 @@ void emit_downsampled(const Blob& lod0, int dimY, int dimZ, int x, int z, int ne
     int top = dimY; // elementBounds = dimensions.y >> lod (lod 0)
     for (int run = 0; run < h.runCount; run++) {
         Run e; memcpy(&e, base + 1 + run, 4);
-        int bottom = top - e.length;
+        // the 16 bits of Length as the count finalize_column wrote: a run of 32768 voxels (a full column of a 32768-high world)
+        // is stored as int16 -32768
+        const int length = (uint16_t)e.length;
+        int bottom = top - length;
         if (e.colorsIndex >= 0)
-            for (int i = 0; i < e.length; i++) acc.add((bottom + i) >> nextLod, colors[e.colorsIndex + e.length - i - 1]);
+            for (int i = 0; i < length; i++) acc.add((bottom + i) >> nextLod, colors[e.colorsIndex + length - i - 1]);
         top = bottom;
     }
 }

@@ -43,8 +43,8 @@ __device__ __forceinline__ V3 cross3(V3 a, V3 b) { return {a.y * b.z - a.z * b.y
 __device__ __forceinline__ V3 normalize3(V3 a) { float r = 1.0f / sqrtf(dot3(a, a)); return a * r; }
 __device__ __forceinline__ int clampi(int x, int a, int b) { return max(a, min(b, x)); }
 __device__ __forceinline__ int f2i_x64(float f) { if (!(f >= -2147483648.0f && f < 2147483648.0f)) return INT_MIN; return (int)f; } // cvttss2si
-__device__ __forceinline__ uint32_t to_byte(float c) { // Color -> Color32: round(clamp01(c) * 255), half to even
-    float v = c < 0.0f ? 0.0f : (c > 1.0f ? 1.0f : c);
+__device__ __forceinline__ uint32_t to_byte(float c) { // Color -> Color32: round(clamp01(c) * 255), half to even; NaN -> 0
+    float v = c > 0.0f ? (c < 1.0f ? c : 1.0f) : 0.0f;
     return (uint32_t)rintf(v * 255.0f) & 0xffu;
 }
 
@@ -69,6 +69,7 @@ __device__ void tri_setup(const float* __restrict__ xyz, const uint8_t* __restri
     a = a + normalize3(a - mid) * 0.5f;   // corners pushed outwards by half a voxel (:44-46)
     b = b + normalize3(b - mid) * 0.5f;
     c = c + normalize3(c - mid) * 0.5f;
+    // fminf / fmaxf ignore a NaN corner (math.min / math.max of the reference; DESIGN.md §3.4)
     V3 mn = {fminf(a.x, fminf(b.x, c.x)), fminf(a.y, fminf(b.y, c.y)), fminf(a.z, fminf(b.z, c.z))};
     V3 mxv = {fmaxf(a.x, fmaxf(b.x, c.x)), fmaxf(a.y, fmaxf(b.y, c.y)), fmaxf(a.z, fmaxf(b.z, c.z))};
     t.lo[0] = clampi(f2i_x64(floorf(mn.x)), 0, mx); t.lo[1] = clampi(f2i_x64(floorf(mn.y)), 0, my); t.lo[2] = clampi(f2i_x64(floorf(mn.z)), 0, mz);

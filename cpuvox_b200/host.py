@@ -259,7 +259,9 @@ class RenderManager:
         dims, vox = (C.c_int32 * 3)(), (C.c_int64 * LOD_LEVELS)()
         self._ck(lib.cvx_world_build_from_mesh(self._ctx, _ptr(positions), _ptr(colors32), positions.shape[0], max_dimension, C.byref(fl), lods,
                                                C.byref(dims), C.byref(vox)))
-        self.world = World((dims[0], dims[1], dims[2]), [], [], [int(v) for v in vox][:lods])
+        # the build stops at the first LOD where an axis reaches 0, as World._from_builder does
+        built = next((lod for lod in range(lods) if min(dims[0] >> lod, dims[1] >> lod, dims[2] >> lod) < 1), lods)
+        self.world = World((dims[0], dims[1], dims[2]), [], [], [int(v) for v in vox][:built])
         self._refresh_lods()
         return self.world
 

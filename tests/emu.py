@@ -23,6 +23,7 @@ def lib():
         L.emu_world_create.argtypes = [C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]
         L.emu_world_destroy.argtypes = [C.c_void_p]
         L.emu_world_regular.argtypes = [C.c_void_p]
+        L.emu_transcode_verdict.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int)]
         L.emu_phase1.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 5
         _lib = L
     return _lib
@@ -47,6 +48,14 @@ class EmuWorld:
         if getattr(self, "_w", None):
             lib().emu_world_destroy(self._w)
             self._w = None
+
+
+def transcode_verdict(blob: np.ndarray, column_count: int, dims, lod: int = 0):
+    """world_transcode.h on one LOD blob: (accepted, first bad column or -1, regular)."""
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    bad, regular = C.c_int64(-1), C.c_int(0)
+    ok = lib().emu_transcode_verdict(blob.ctypes.data, blob.nbytes, column_count, lod, (C.c_int32 * 3)(*dims), C.byref(bad), C.byref(regular))
+    return bool(ok), int(bad.value), bool(regular.value)
 
 
 def render_raybuffers(world: EmuWorld, setup, W, H, variant=0, group=32, counters=True, fill=0, threads=0, ray_begin=0, ray_end=-1):

@@ -18,35 +18,32 @@ def encode_world(grid: np.ndarray, lod: int = 0):
     assert cc >= dx * dz
     headers = np.zeros((cc, 3), dtype=np.uint32)
     cells = []
-    for x in range(dx):
-        for z in range(dz):
-            col = grid[x, :, z]
-            if not col.any():
-                continue
-            runs, colors = [], []
-            y = dy - 1
-            while y >= 0:  # top -> bottom
-                solid = col[y] != 0
-                y0 = y
-                while y >= 0 and (col[y] != 0) == solid:
-                    y -= 1
-                length = y0 - y
-                if solid:
-                    runs.append((len(colors), length))
-                    colors.extend(int(c) for c in col[y + 1:y0 + 1][::-1])
-                else:
-                    runs.append((-1, length))
-            ys = np.nonzero(col)[0]
-            off = len(cells)
-            cells.append(0)
-            for ci, ln in runs:
-                cells.append((ci & 0xFFFF) | ((ln & 0xFFFF) << 16))
-            cells.append(0)
-            cells.extend(colors)
-            idx = x * dz + z
-            headers[idx, 0] = off
-            headers[idx, 1] = len(runs) | (((int(ys.min())) << lod) << 16)
-            headers[idx, 2] = (int(ys.max()) + 1) << lod
+    for x, z in zip(*np.nonzero(grid.any(axis=1))):  # the non-empty columns, in index order
+        col = grid[x, :, z]
+        runs, colors = [], []
+        y = dy - 1
+        while y >= 0:  # top -> bottom
+            solid = col[y] != 0
+            y0 = y
+            while y >= 0 and (col[y] != 0) == solid:
+                y -= 1
+            length = y0 - y
+            if solid:
+                runs.append((len(colors), length))
+                colors.extend(int(c) for c in col[y + 1:y0 + 1][::-1])
+            else:
+                runs.append((-1, length))
+        ys = np.nonzero(col)[0]
+        off = len(cells)
+        cells.append(0)
+        for ci, ln in runs:
+            cells.append((ci & 0xFFFF) | ((ln & 0xFFFF) << 16))
+        cells.append(0)
+        cells.extend(colors)
+        idx = x * dz + z
+        headers[idx, 0] = off
+        headers[idx, 1] = len(runs) | (((int(ys.min())) << lod) << 16)
+        headers[idx, 2] = (int(ys.max()) + 1) << lod
     if not cells:
         cells = [0]
     blob = np.concatenate([headers.reshape(-1).view(np.uint8), np.array(cells, dtype=np.uint32).view(np.uint8)])

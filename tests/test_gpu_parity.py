@@ -596,11 +596,13 @@ def test_gpu_world_builder_matches_host_builder(cv, rm):
         dev = rm.build_world_from_obj(MILL, maxdim)
         t2 = time.perf_counter()
         assert dev.dims == host.dims and dev.column_counts == host.column_counts and dev.voxel_counts == host.voxel_counts
+        assert len(dev.blobs) == len(host.blobs)
         for lod, (a, b) in enumerate(zip(dev.blobs, host.blobs)):
             assert a.nbytes == b.nbytes, f"mill {maxdim} LOD {lod}: blob sizes {a.nbytes} != {b.nbytes}"
             assert np.array_equal(a, b), f"mill {maxdim} LOD {lod}: {int((a != b).sum())} bytes differ"
         print(f"mill {maxdim}^3: host builder {t1 - t0:.3f} s, device builder {t2 - t1:.3f} s (incl. blob download), {host.voxel_counts[0]} voxels")
-    # a random triangle soup with random vertex colours, non-cubic dimensions, all three flips
+    # a random triangle soup with random vertex colours, no flip and all three flips. Its triangles lie in the unit cube, so the
+    # world is 256^3; non-cubic worlds and the other edges are in test_world_production.py
     rng = np.random.default_rng(17)
     pos = rng.uniform(0.0, 1.0, size=(300 * 3, 3)).astype(np.float32) * np.array([1.0, 0.45, 0.7], dtype=np.float32)
     tri_c = rng.uniform(0.0, 1.0, size=(300, 1, 3)).astype(np.float32)
@@ -610,7 +612,7 @@ def test_gpu_world_builder_matches_host_builder(cv, rm):
     for flips in ((False, False, False), (True, True, True)):
         host = cv.World.from_mesh(pos, col, 200, flips=flips)
         dev = rm.build_world_from_mesh(pos, col, 200, flips=flips)
-        assert dev.dims == host.dims and dev.voxel_counts == host.voxel_counts
+        assert dev.dims == host.dims and dev.voxel_counts == host.voxel_counts and len(dev.blobs) == len(host.blobs) == 6
         for lod, (a, b) in enumerate(zip(dev.blobs, host.blobs)):
             assert np.array_equal(a, b), f"soup flips {flips} LOD {lod}"
     # mesh -> resident world without leaving the device (cvx_world_build_from_mesh): frames equal those of the uploaded host-built world

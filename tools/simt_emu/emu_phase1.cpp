@@ -70,6 +70,18 @@ emu_world* emu_world_create(int lods, const int32_t dims[3], const void* const* 
     return w;
 }
 
+// The host transcode's verdict on one LOD blob, as cvx_world_upload would be given it: returns 1 when it accepts the blob, 0 when it
+// rejects it (*bad_column = the first column pointing outside the element area); *regular = the LOD's boundary-table flag.
+int emu_transcode_verdict(const void* blob, int64_t bytes, int32_t column_count, int lod, const int32_t dims[3], int64_t* bad_column, int* regular) {
+    const int64_t needCols = (int64_t)(dims[0] >> lod) * (dims[2] >> lod);
+    const int64_t cells = (bytes - 12 * (int64_t)column_count) / 4;
+    cvxh_lod_tables t;
+    const bool ok = cvxh_transcode_lod(blob, needCols, column_count, cells, lod, dims[1], t);
+    *bad_column = t.bad_column;
+    *regular = t.regular ? 1 : 0;
+    return ok ? 1 : 0;
+}
+
 #ifdef CVX_EMU_STATS
 void emu_set_stats(unsigned long long* p) { emu_stats = p; } // 16 counters per flat ray
 #endif
