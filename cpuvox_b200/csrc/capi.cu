@@ -135,14 +135,7 @@ int validate_setup(cvx_ctx* ctx, const cvx_frame_setup* s, int total) {
 
 void make_frame(cvx_ctx* ctx, const cvx_frame_setup* s, cvxd_frame& f) {
     cvxh::frame_from_setup(s, ctx->width, ctx->height, f);
-    cvxd_frame_set_world(&f, &ctx->world);
-    // The reference indexes worldLODs / LODDistances unchecked (DrawSegmentRayJob.cs:123-128,237-243): a ray that passes
-    // LODDistances[lod] moves on to LOD lod + 1 whether or not it exists. Here the last uploaded LOD of the contiguous run from
-    // LOD 0 is never left: its distance and the ones after it are +inf (identical to the reference whenever the reference is
-    // well defined, i.e. every LOD a ray can reach exists and LODDistances[5] lies beyond the far clip, as SetupLods makes it).
-    int last = 0;
-    while (last + 1 < CVXD_LODS && ctx->world.lods[last + 1].headers) last++;
-    for (int i = last; i < CVXD_LODS; i++) f.lod_dist[i] = __builtin_inff();
+    cvxd_frame_set_world(&f, &ctx->world); // also sets the distances of the last uploaded LOD and beyond to +inf
     f.td = ctx->td; f.lr = ctx->lr;
     f.counters = (ctx->flags & CVX_FLAG_COUNTERS) ? ctx->counters : nullptr;
     f.general_path = ctx->generalPath;

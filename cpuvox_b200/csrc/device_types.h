@@ -115,7 +115,16 @@ static inline void cvxd_blit_prepare(cvxd_blit* b) {
     }
 }
 
-static inline void cvxd_frame_set_world(cvxd_frame* f, const cvxd_world* w) { f->cam_y_norm = f->pos_y / w->dim_y_f; }
+/* The reference indexes worldLODs / LODDistances unchecked (DrawSegmentRayJob.cs:123-128,237-243): a ray that passes LODDistances[lod]
+ * moves on to LOD lod + 1 whether or not it exists. Here the last uploaded LOD of the contiguous run from LOD 0 is never left: its
+ * distance and the ones after it are +inf (identical to the reference whenever the reference is well defined, i.e. every LOD a ray
+ * can reach exists and LODDistances[5] lies beyond the far clip, as SetupLods makes it). */
+static inline void cvxd_frame_set_world(cvxd_frame* f, const cvxd_world* w) {
+    f->cam_y_norm = f->pos_y / w->dim_y_f;
+    int last = 0;
+    while (last + 1 < CVXD_LODS && w->lods[last + 1].headers) last++;
+    for (int i = last; i < CVXD_LODS; i++) f->lod_dist[i] = __builtin_inff();
+}
 
 struct cvxd_ray_state { /* mirrors cvx_ray_state */
     int32_t segment, plane_ray_index, status, lod;

@@ -52,8 +52,9 @@ __device__ __forceinline__ float lerpf(float a, float b, float t) { return a + t
 __device__ __forceinline__ float unlerpf(float a, float b, float x) { return (x - a) / (b - a); }
 __device__ __forceinline__ F3 lerp3(F3 a, F3 b, float t) { return F3{lerpf(a.x, b.x, t), lerpf(a.y, b.y, t), lerpf(a.z, b.z, t)}; }
 __device__ __forceinline__ float signf(float x) { return (float)((x > 0.0f ? 1 : 0) - (x < 0.0f ? 1 : 0)); }
-__device__ __forceinline__ float minf_(float a, float b) { return a < b ? a : b; }
-__device__ __forceinline__ float maxf_(float a, float b) { return a > b ? a : b; }
+// math.min / math.max as the reference build pins them (Unity.Mathematics): a NaN second operand gives the first, a tie (±0) the second
+__device__ __forceinline__ float minf_(float a, float b) { return (b != b || a < b) ? a : b; }
+__device__ __forceinline__ float maxf_(float a, float b) { return (b != b || a > b) ? a : b; }
 // (int)float as x64 cvttss2si: NaN / out of range -> INT_MIN
 __device__ __forceinline__ int f2i(float f) { const int r = __float2int_rz(f); return f < 2147483648.0f ? r : (int)0x80000000; } // cvt saturates low; NaN/high -> INT_MIN
 __device__ __forceinline__ float float_epsilon() { return __int_as_float(1); }
@@ -79,8 +80,10 @@ __device__ __forceinline__ void dda_init(Dda& d, float sx, float sz, float dx, f
 }
 
 __device__ __forceinline__ void dda_next_lod(Dda& d, int voxelSize) { // :31-73
+    const float ninf = __int_as_float(0xff800000), pinf = __int_as_float(0x7f800000);
     int rx = d.px & (voxelSize * 2 - 1), rz = d.pz & (voxelSize * 2 - 1);
-    float prevx = d.tmx - d.tdx, prevz = d.tmz - d.tdz;
+    // a still axis entered from outside has tMax = +inf (dda_step_to_world): its last crossing stays -inf, tMax - tDelta would be +inf
+    float prevx = d.tmx != pinf ? d.tmx - d.tdx : ninf, prevz = d.tmz != pinf ? d.tmz - d.tdz : ninf;
     if ((d.dir_x >= 0.0f) == (rx < voxelSize)) d.tmx += d.tdx; else prevx -= d.tdx;
     if ((d.dir_z >= 0.0f) == (rz < voxelSize)) d.tmz += d.tdz; else prevz -= d.tdz;
     d.dl = maxf_(prevx, prevz);
@@ -112,15 +115,20 @@ __device__ bool dda_step_to_world(Dda& d, float dimX, float dimZ) { // StepToWor
         hit = d.dir_x > 0.0f ? floorf(hit) : ceilf(hit);
         off = hit - d.start_x;
         lastx = off / d.dir_x;
-    } else {
+    } else if (d.dir_z != 0.0f) {
         lastx = tminx;
         float off = tmint * d.dir_z;
         float hit = d.start_z + off;
         hit = d.dir_z > 0.0f ? floorf(hit) : ceilf(hit);
         off = hit - d.start_z;
         lastz = off / d.dir_z;
+    } else {
+        lastx = tminx; lastz = ninf;
     }
-    d.tmx = lastx + d.tdx; d.tmz = lastz + d.tdz;
+    // Still-axis rule (DESIGN.md §5): an axis with dir == 0 never bounds the entry and is never crossed, tLast = -inf and tMax = +inf.
+    // The reference divides by the zero component here (a NaN or +inf last distance for a still z, tMax = -inf for a still x).
+    d.tmx = d.dir_x != 0.0f ? lastx + d.tdx : pinf;
+    d.tmz = d.dir_z != 0.0f ? lastz + d.tdz : pinf;
     d.dl = maxf_(lastx, lastz);
     d.dn = minf_(d.tmx, d.tmz);
     float mid = lerpf(d.dl, d.dn, 0.5f);
@@ -192,8 +200,11 @@ __device__ void setup_ray(const cvxd_world& world, const cvxd_frame& f, int flat
     if (rs.dda.px < 0 || rs.dda.pz < 0 || rs.dda.px >= world.dim_x || rs.dda.pz >= world.dim_z) {
         rs.status = 1;
         if (dda_step_to_world(rs.dda, (float)world.dim_x, (float)world.dim_z)) {
+            // never past the last LOD of the contiguous run uploaded from LOD 0 (the reference indexes worldLODs unchecked)
+            int lastLod = 0;
+            while (lastLod + 1 < CVXD_LODS && world.lods[lastLod + 1].headers) lastLod++;
             float lodMax = f.lod_dist[0];
-            while (rs.dda.dl >= lodMax) {
+            while (rs.lod < lastLod && rs.dda.dl >= lodMax) {
                 dda_next_lod(rs.dda, 1 << rs.lod);
                 rs.lod++;
                 rs.lod_steps++;
@@ -415,7 +426,10 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
             // Z[b] likewise (ties go to z). The two chains are accumulated serially (same float additions as the reference), lane j
             // keeps X[j] and Z[j]; lane k then finds by a merge-path binary search how many of its first k steps were x steps —
             // a_k = the largest a with X[a-1] < Z[k-a] — which gives its cell, its last/next distances and its header address.
-            if (ray.dl >= lodMax) { // :237-243, tested once per visited cell: here for cell 0, for later cells by cutting the batch
+            // :237-243, tested once per visited cell: here for cell 0, for later cells by cutting the batch. This needs no LOD bound:
+            // lod_dist of the last uploaded LOD is +inf (cvxd_frame_set_world), and dl is never +inf here, since every dl is a finite
+            // crossing distance, a still axis contributes -inf (dda_step_to_world, dda_next_lod) and a NaN compares false.
+            if (ray.dl >= lodMax) {
                 dda_next_lod(ray, voxelScale);
                 lod++; voxelScale *= 2;
                 lodMax = f.lod_dist[lod];

@@ -37,8 +37,10 @@ inline float m_lerp(float a, float b, float t) { return a + t * (b - a); }
 inline float m_unlerp(float a, float b, float x) { return (x - a) / (b - a); }
 inline f3 m_lerp3(f3 a, f3 b, float t) { return {m_lerp(a.x, b.x, t), m_lerp(a.y, b.y, t), m_lerp(a.z, b.z, t)}; }
 inline float m_sign(float x) { return (float)((x > 0.0f ? 1 : 0) - (x < 0.0f ? 1 : 0)); }
-inline float m_min(float a, float b) { return a < b ? a : b; }   // math.min: select(a,b, b<a) – same for non-NaN
-inline float m_max(float a, float b) { return a > b ? a : b; }
+// math.min / math.max as the reference build pins them (unity_shim.hpp: isnan(y) || x < y ? x : y): a NaN second operand gives the
+// first, a tie (±0) gives the second
+inline float m_min(float a, float b) { return (std::isnan(b) || a < b) ? a : b; }
+inline float m_max(float a, float b) { return (std::isnan(b) || a > b) ? a : b; }
 inline int i_min(int a, int b) { return a < b ? a : b; }
 inline int i_max(int a, int b) { return a > b ? a : b; }
 inline int i_clamp(int x, int a, int b) { return i_max(a, i_min(b, x)); }
@@ -248,6 +250,7 @@ struct WorldLod {
 struct orc_world {
     int dimX, dimY, dimZ;
     WorldLod lods[ORC_LOD_LEVELS];
+    int lastLod = 0; // last LOD of the contiguous run set from LOD 0: rays never switch past it
 };
 
 namespace {
@@ -285,7 +288,8 @@ struct DDA {
     void next_lod(int currentVoxelSize) {
         int rx = position.x & (currentVoxelSize * 2 - 1);
         int ry = position.y & (currentVoxelSize * 2 - 1);
-        f2 prev = {tMax.x - tDelta.x, tMax.y - tDelta.y};
+        // a still axis entered from outside has tMax = +inf (step_to_world_intersection): its last crossing stays -inf
+        f2 prev = {tMax.x != INFINITY ? tMax.x - tDelta.x : -INFINITY, tMax.y != INFINITY ? tMax.y - tDelta.y : -INFINITY};
         if (dir.x >= 0.0f) { if (rx < currentVoxelSize) tMax.x += tDelta.x; else prev.x -= tDelta.x; }
         else               { if (rx < currentVoxelSize) prev.x -= tDelta.x; else tMax.x += tDelta.x; }
         if (dir.y >= 0.0f) { if (ry < currentVoxelSize) tMax.y += tDelta.y; else prev.y -= tDelta.y; }
@@ -317,15 +321,18 @@ struct DDA {
             hit = dir.x > 0.0f ? floorf(hit) : ceilf(hit);
             off = hit - start.x;
             tLast.x = off / dir.x;
-        } else {
+        } else if (dir.y != 0.0f) {
             tLast.x = tmin.x;
             float off = tmint * dir.y;
             float hit = start.y + off;
             hit = dir.y > 0.0f ? floorf(hit) : ceilf(hit);
             off = hit - start.y;
             tLast.y = off / dir.y;
+        } else {
+            tLast = {tmin.x, -INFINITY};
         }
-        tMax = {tLast.x + tDelta.x, tLast.y + tDelta.y};
+        // still-axis rule (DESIGN.md §5): an axis with dir == 0 never bounds the entry and is never crossed (tLast -inf, tMax +inf)
+        tMax = {dir.x != 0.0f ? tLast.x + tDelta.x : INFINITY, dir.y != 0.0f ? tLast.y + tDelta.y : INFINITY};
         dist = {m_max(tLast.x, tLast.y), m_min(tMax.x, tMax.y)};
         float mid = m_lerp(dist.x, dist.y, 0.5f);
         position = {f2i(floorf(start.x + mid * dir.x)), f2i(floorf(start.y + mid * dir.y))};
@@ -531,7 +538,7 @@ bool setup_ray(const orc_world* w, const orc_frame_setup* s, const SegCtx ctx[4]
     i2 sp = cont.dda.position;
     if (sp.x < 0 || sp.y < 0 || sp.x >= w->dimX || sp.y >= w->dimZ) {
         if (cont.dda.step_to_world_intersection(f2{(float)w->dimX, (float)w->dimZ})) {
-            while (cont.dda.dist.x >= lodMax) {
+            while (cont.lod < w->lastLod && cont.dda.dist.x >= lodMax) { // never past the last uploaded LOD
                 cont.dda.next_lod(1 << cont.lod);
                 cont.lod++;
                 cn.dda_steps++;
@@ -598,7 +605,7 @@ void execute_ray(const orc_world* w, const SegCtx& sc, const Cam& cam, const Ray
     auto madd3 = [](f3 a, f3 d, float t) { return f3{a.x + d.x * t, a.y + d.y * t, a.z + d.z * t}; };
 
     while (true) {
-        if (ray.dist.x >= lodMax) { // :237-243
+        if (lod < w->lastLod && ray.dist.x >= lodMax) { // :237-243, never past the last uploaded LOD
             ray.next_lod(voxelScale);
             lod++;
             voxelScale *= 2;
@@ -866,10 +873,16 @@ int orc_world_set_lod(orc_world* w, int32_t lod, const void* blob, int64_t bytes
     l.elements = (const RLEElement*)(l.columns + column_count);
     l.lod = lod;
     l.indexingMulX = w->dimZ >> lod;
+    w->lastLod = 0;
+    while (w->lastLod + 1 < ORC_LOD_LEVELS && w->lods[w->lastLod + 1].blob) w->lastLod++;
     return 0;
 }
 
 void orc_world_free(orc_world* w) { delete w; }
+
+void orc_min_max(const float* a, const float* b, int32_t n, float* out_min, float* out_max) {
+    for (int32_t i = 0; i < n; i++) { out_min[i] = m_min(a[i], b[i]); out_max[i] = m_max(a[i], b[i]); }
+}
 
 int orc_hardware_threads(void) { int n = (int)std::thread::hardware_concurrency(); return n > 0 ? n : 1; }
 

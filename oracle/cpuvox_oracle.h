@@ -84,6 +84,8 @@ typedef struct orc_world orc_world;
 orc_world* orc_world_create(int32_t dim_x, int32_t dim_y, int32_t dim_z);
 int orc_world_set_lod(orc_world* w, int32_t lod, const void* blob, int64_t bytes, int32_t column_count);
 void orc_world_free(orc_world* w);
+/* math.min / math.max of the renderer, elementwise (test hook for the NaN and signed-zero rule) */
+void orc_min_max(const float* a, const float* b, int32_t n, float* out_min, float* out_max);
 
 void orc_quat_euler(float x_deg, float y_deg, float z_deg, float out_quat[4]);
 void orc_limit_rotation_horizon(orc_pose* pose);

@@ -70,6 +70,7 @@ def lib():
         L.orc_world_create.argtypes = [C.c_int32] * 3
         L.orc_world_set_lod.argtypes = [P, C.c_int32, P, C.c_int64, C.c_int32]
         L.orc_world_free.argtypes = [P]
+        L.orc_min_max.argtypes = [P, P, C.c_int32, P, P]
         L.orc_quat_euler.argtypes = [C.c_float] * 3 + [C.POINTER(C.c_float * 4)]
         L.orc_limit_rotation_horizon.argtypes = [C.POINTER(Pose)]
         L.orc_setup_lods.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float, C.POINTER(C.c_float * LODS)]
@@ -192,6 +193,15 @@ def ray_setup(world: OracleWorld, setup: FrameSetup, width, height) -> np.ndarra
     n = lib().orc_ray_setup(world._w, C.byref(setup), width, height, out.ctypes.data_as(C.c_void_p), total)
     assert n == total
     return out[:total]
+
+
+def min_max(a, b):
+    """The renderer's math.min / math.max, elementwise over float32 arrays: (min, max)."""
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    b = np.ascontiguousarray(b, dtype=np.float32)
+    mn, mx = np.empty_like(a), np.empty_like(a)
+    lib().orc_min_max(a.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), a.size, mn.ctypes.data_as(C.c_void_p), mx.ctypes.data_as(C.c_void_p))
+    return mn, mx
 
 
 def dda_walk(start, direction, lod_distances, far_clip, max_steps=100000):

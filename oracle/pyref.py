@@ -42,6 +42,16 @@ def unlerp(a, b, x):
     return (x - a) / (b - a)
 
 
+def umin(x, y):
+    """math.min as the reference build pins it (Unity.Mathematics): isnan(y) || x < y ? x : y. A NaN y gives x, a tie (±0) gives y."""
+    return x if (np.isnan(y) or x < y) else y
+
+
+def umax(x, y):
+    """math.max: isnan(y) || x > y ? x : y."""
+    return x if (np.isnan(y) or x > y) else y
+
+
 def sign(x):
     return F(1.0) if x > F(0) else (F(-1.0) if x < F(0) else F(0.0))
 
@@ -79,16 +89,17 @@ class DDA:
         self.start, self.dir = (F(start[0]), F(start[1])), (F(direction[0]), F(direction[1]))
         fl = (np.floor(self.start[0]), np.floor(self.start[1]))
         self.position = [to_int(fl[0]), to_int(fl[1])]
-        self.t_delta = [F(1.0) / max(F(0.0000001), abs(self.dir[0])), F(1.0) / max(F(0.0000001), abs(self.dir[1]))]
+        self.t_delta = [F(1.0) / umax(F(0.0000001), abs(self.dir[0])), F(1.0) / umax(F(0.0000001), abs(self.dir[1]))]
         sd = (sign(self.dir[0]), sign(self.dir[1]))
         self.step = [to_int(sd[0]), to_int(sd[1])]
         frac = (self.start[0] - fl[0], self.start[1] - fl[1])
         self.t_max = [(sd[k] * -frac[k] + (sd[k] * F(0.5)) + F(0.5)) * self.t_delta[k] for k in range(2)]
-        self.dist = [max(self.t_max[0] - self.t_delta[0], self.t_max[1] - self.t_delta[1]), min(self.t_max[0], self.t_max[1])]
+        self.dist = [umax(self.t_max[0] - self.t_delta[0], self.t_max[1] - self.t_delta[1]), umin(self.t_max[0], self.t_max[1])]
 
     def next_lod(self, size):                                      # :31-73
         rem = [self.position[0] & (size * 2 - 1), self.position[1] & (size * 2 - 1)]
-        prev = [self.t_max[0] - self.t_delta[0], self.t_max[1] - self.t_delta[1]]
+        # a still axis entered from outside has t_max = +inf (step_to_world_intersection): its last crossing stays -inf
+        prev = [self.t_max[k] - self.t_delta[k] if self.t_max[k] != POS_INF else NEG_INF for k in range(2)]
         for k in range(2):
             if self.dir[k] >= F(0):
                 if rem[k] < size:
@@ -100,7 +111,7 @@ class DDA:
                     prev[k] = prev[k] - self.t_delta[k]
                 else:
                     self.t_max[k] = self.t_max[k] + self.t_delta[k]
-        self.dist = [max(prev[0], prev[1]), min(self.t_max[0], self.t_max[1])]
+        self.dist = [umax(prev[0], prev[1]), umin(self.t_max[0], self.t_max[1])]
         self.position = [self.position[0] - rem[0], self.position[1] - rem[1]]
         self.t_delta = [self.t_delta[0] * F(2.0), self.t_delta[1] * F(2.0)]
         self.step = [self.step[0] * 2, self.step[1] * 2]
@@ -114,8 +125,8 @@ class DDA:
             if self.dir[k] != F(0):
                 t1 = -self.start[k] * inv[k]
                 t2 = (dims[k] - self.start[k]) * inv[k]
-                tmin[k], tmax[k] = min(t1, t2), max(t1, t2)
-        tmint, tmaxt = max(tmin[0], tmin[1]), min(tmax[0], tmax[1])
+                tmin[k], tmax[k] = umin(t1, t2), umax(t1, t2)
+        tmint, tmaxt = umax(tmin[0], tmin[1]), umin(tmax[0], tmax[1])
         if tmaxt < tmint or tmint <= F(0):
             return False
         t_last = [F(0), F(0)]
@@ -124,13 +135,17 @@ class DDA:
         else:
             a, o = 1, 0
         t_last[o] = tmin[o]
-        offset = tmint * self.dir[a]
-        hit = self.start[a] + offset
-        hit = np.floor(hit) if self.dir[a] > F(0) else np.ceil(hit)
-        offset = hit - self.start[a]
-        t_last[a] = offset / self.dir[a]
-        self.t_max = [t_last[0] + self.t_delta[0], t_last[1] + self.t_delta[1]]
-        self.dist = [max(t_last[0], t_last[1]), min(self.t_max[0], self.t_max[1])]
+        if self.dir[a] != F(0):
+            offset = tmint * self.dir[a]
+            hit = self.start[a] + offset
+            hit = np.floor(hit) if self.dir[a] > F(0) else np.ceil(hit)
+            offset = hit - self.start[a]
+            t_last[a] = offset / self.dir[a]
+        else:
+            t_last[a] = NEG_INF
+        # still-axis rule (DESIGN.md §5): an axis with dir == 0 never bounds the entry and is never crossed (t_last -inf, t_max +inf)
+        self.t_max = [t_last[k] + self.t_delta[k] if self.dir[k] != F(0) else POS_INF for k in range(2)]
+        self.dist = [umax(t_last[0], t_last[1]), umin(self.t_max[0], self.t_max[1])]
         mid = lerp(self.dist[0], self.dist[1], F(0.5))
         self.position = [to_int(np.floor(self.start[0] + mid * self.dir[0])), to_int(np.floor(self.start[1] + mid * self.dir[1]))]
         return True
@@ -144,11 +159,11 @@ class DDA:
             crossed = self.t_max[1]
             self.t_max[1] = self.t_max[1] + self.t_delta[1]
             self.position[1] += self.step[1]
-        self.dist = [crossed, min(self.t_max[0], self.t_max[1])]
+        self.dist = [crossed, umin(self.t_max[0], self.t_max[1])]
         return crossed >= farclip
 
     def is_beyond_far_clip(self, farclip):                         # :152-155
-        return min(self.t_max[0], self.t_max[1]) >= farclip
+        return umin(self.t_max[0], self.t_max[1]) >= farclip
 
 
 # ---- CameraData helpers ------------------------------------------------------------------------------------------------------
@@ -249,7 +264,9 @@ def render_raybuffers(worlds, setup, W, H, ray_indices=None):
     m = [F(v) for v in cam.world_to_screen]
     pos_xz, pos_y = (F(cam.position_xz[0]), F(cam.position_xz[1])), F(cam.position_y)
     far_clip = F(cam.far_clip)
-    lod_dist = [F(v) for v in cam.lod_distances]
+    # a ray never switches past the last LOD given: its distance and the ones after it are +inf
+    lod_dist = [F(v) if k < len(worlds) - 1 else POS_INF for k, v in enumerate(cam.lod_distances)]
+    last_lod = len(worlds) - 1
     inverse = bool(cam.inverse_element_iteration_direction)
     total = sum(max(0, c["ray_count"]) for c in ctx)
     with np.errstate(all="ignore"):
@@ -281,7 +298,7 @@ def render_raybuffers(worlds, setup, W, H, ray_indices=None):
             if ray.position[0] < 0 or ray.position[1] < 0 or ray.position[0] >= w0.dims[0] or ray.position[1] >= w0.dims[2]:
                 if ray.step_to_world_intersection(w0.dims[0], w0.dims[2]):
                     lod_max = lod_dist[0]
-                    while ray.dist[0] >= lod_max:
+                    while lod < last_lod and ray.dist[0] >= lod_max:
                         ray.next_lod(1 << lod)
                         lod += 1
                         lod_max = lod_dist[lod]
@@ -340,7 +357,7 @@ def execute_ray(worlds, seg, ray, lod, row, m, pos_y, far_clip, lod_dist, ITER, 
         return b_min, b_max
 
     while True:
-        if ray.dist[0] >= lod_max:                            # :237-243
+        if lod < len(worlds) - 1 and ray.dist[0] >= lod_max:  # :237-243, never past the last LOD given
             ray.next_lod(voxel_scale)
             lod += 1
             voxel_scale *= 2
@@ -414,8 +431,7 @@ def execute_ray(worlds, seg, ray, lod, row, m, pos_y, far_clip, lod_dist, ITER, 
                     max_n, min_n = min_n, max_n
                 if max_l < min_l:
                     max_l, min_l = min_l, max_l
-                c_min = min_l if min_l < min_n else min_n      # math.min / math.max
-                c_max = max_l if max_l > max_n else max_n
+                c_min, c_max = umin(min_l, min_n), umax(max_l, max_n)
             wb_min, wb_max = np.floor(wb_min), np.ceil(wb_max)
             wr_min, wr_max = to_int(np.floor(c_min)), to_int(np.ceil(c_max))
             if wr_max < nf_min or wr_min > nf_max:
@@ -556,7 +572,7 @@ def blit(setup, W, H, td, lr):
             if det < 0:
                 b, c = -b, -c
             inside = (b >= 0) & (c >= 0) & ~done
-            sc = np.minimum(b, c) / np.abs(det)
+            sc = np.where(np.isnan(c) | (b < c), b, c) / np.abs(det)   # math.min
             better = ~done & ~inside & (sc > score)
             take = inside | better
             best[take] = k

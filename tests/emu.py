@@ -24,6 +24,7 @@ def lib():
         L.emu_world_destroy.argtypes = [C.c_void_p]
         L.emu_world_regular.argtypes = [C.c_void_p]
         L.emu_transcode_verdict.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int)]
+        L.emu_min_max.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.emu_phase1.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 5
         _lib = L
     return _lib
@@ -56,6 +57,15 @@ def transcode_verdict(blob: np.ndarray, column_count: int, dims, lod: int = 0):
     bad, regular = C.c_int64(-1), C.c_int(0)
     ok = lib().emu_transcode_verdict(blob.ctypes.data, blob.nbytes, column_count, lod, (C.c_int32 * 3)(*dims), C.byref(bad), C.byref(regular))
     return bool(ok), int(bad.value), bool(regular.value)
+
+
+def min_max(a, b):
+    """The Phase-1 kernel's minf_ / maxf_, elementwise over float32 arrays: (min, max)."""
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    b = np.ascontiguousarray(b, dtype=np.float32)
+    mn, mx = np.empty_like(a), np.empty_like(a)
+    lib().emu_min_max(a.ctypes.data, b.ctypes.data, a.size, mn.ctypes.data, mx.ctypes.data)
+    return mn, mx
 
 
 def render_raybuffers(world: EmuWorld, setup, W, H, variant=0, group=32, counters=True, fill=0, threads=0, ray_begin=0, ray_end=-1):

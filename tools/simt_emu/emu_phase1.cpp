@@ -82,6 +82,11 @@ int emu_transcode_verdict(const void* blob, int64_t bytes, int32_t column_count,
     return ok ? 1 : 0;
 }
 
+// The kernel's minf_ / maxf_, elementwise (test hook for the NaN and signed-zero rule).
+void emu_min_max(const float* a, const float* b, int n, float* out_min, float* out_max) {
+    for (int i = 0; i < n; i++) { out_min[i] = minf_(a[i], b[i]); out_max[i] = maxf_(a[i], b[i]); }
+}
+
 #ifdef CVX_EMU_STATS
 void emu_set_stats(unsigned long long* p) { emu_stats = p; } // 16 counters per flat ray
 #endif
