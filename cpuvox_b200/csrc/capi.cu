@@ -34,34 +34,37 @@ static_assert(sizeof(cvx_ray_hit) == sizeof(cvxd_ray_hit) && sizeof(cvx_ray_hit)
 
 extern "C" int cvx_ring_close(cvx_ctx* ctx);
 
+// cvx_draw_batch keeps several views in flight: view i renders on slot i % slotCount, each slot with its own raybuffers and
+// framebuffer. Slot 0 renders on the context's stream (slot_stream; its own `stream` stays null) and gets its buffers from
+// cvx_set_resolution; the others have a stream of their own and get their buffers on first use.
 struct cvx_slot {
     cudaStream_t stream = nullptr;
     uint32_t* td = nullptr;
     uint32_t* lr = nullptr;
     uint32_t* frame = nullptr;
-    cudaEvent_t done = nullptr;
+    cudaEvent_t done = nullptr;     // slots 1..: joins the slot's views into the context's stream
+};
+
+// device memory of one uploaded LOD (what ctx->world.lods[i] points into)
+struct cvx_lod_memory {
+    void* blob = nullptr;           // the uploaded blob: column headers, then the element area the kernels read
+    void* headers = nullptr;        // the Phase-1 tables built from it (world_builder_gpu.cu)
+    void* bounds = nullptr;
+    bool regular = false;
 };
 
 struct cvx_ctx {
     int device = 0;
     int flags = 0;
     cudaStream_t stream = nullptr;      // compute
-    cudaStream_t copyStream = nullptr;  // (kept for cvx_sync symmetry; frame copies ride on the slot streams)
+    cudaStream_t copyStream = nullptr;  // device->host copies of pooled batch frames (cvx_draw_batch with dst_frames) and cvx_ring_consume
     bool ownStream = true;
     cvxd_world world;
-    void* lodHeaders[CVX_LOD_LEVELS];
-    void* lodElements[CVX_LOD_LEVELS];
-    void* lodBounds[CVX_LOD_LEVELS];
-    bool lodRegular[CVX_LOD_LEVELS];
+    cvx_lod_memory lod[CVX_LOD_LEVELS];
     int width = 0, height = 0;
-    uint32_t* td = nullptr;
-    uint32_t* lr = nullptr;
-    uint32_t* frames[2] = {nullptr, nullptr}; // internal framebuffer (index 0; index 1 unused)
-    // cvx_draw_batch keeps several views in flight: view i renders on slot i % slotCount, each slot a stream with its own
-    // raybuffers and framebuffer. Slot 0 is the context's stream and buffers; the others are allocated on first use.
-    cvx_slot extra[CVX_MAX_SLOTS - 1];
+    cvx_slot slots[CVX_MAX_SLOTS];
     int slotCount = CVX_DEFAULT_SLOTS;  // CVX_OPT_FRAMES_IN_FLIGHT
-    int extraReady = 0;                 // extra slots holding buffers for the current resolution
+    int slotsReady = 0;                 // slots holding buffers for the current resolution
     int lastSlot = 0;                   // slot of the most recent view (what the read functions return)
     cudaEvent_t evBatchStart = nullptr;
     // cvx_draw_batch with dst_frames: Phase 2 writes into a pool of framebuffers that a copy stream drains, so a slot starts its next
@@ -77,10 +80,9 @@ struct cvx_ctx {
     uint32_t* presentStage = nullptr;   // cvx_present with a host destination / cvx_present_jpeg: converted frame (W*H*4 bytes)
     cvxjpeg::Encoder* jpeg = nullptr;   // created by the first cvx_present_jpeg
     std::vector<uint8_t> jpegOut;
-    int frameIndex = 0;
     cvxd_counters* counters = nullptr;
     cudaEvent_t evStart = nullptr, evMid = nullptr, evEnd = nullptr;
-    cudaEvent_t evFrameDone[2] = {nullptr, nullptr}, evCopyDone[2] = {nullptr, nullptr};
+    cudaEvent_t evFrameDone = nullptr, evCopyDone = nullptr;  // a pooled batch: its last view rendered / its copies done
     bool timed = false;
     int64_t launches = 0;
     std::vector<cudaEvent_t> profEvents; // 3 per profiled view: start, mid, end
@@ -115,42 +117,57 @@ int fail(cvx_ctx* ctx, int code, const char* fmt, ...) {
 #define CU(ctx, call)                                                                                     \
     do {                                                                                                  \
         cudaError_t e_ = (call);                                                                          \
-        if (e_ != cudaSuccess)                                                                            \
-            return fail(ctx, e_ == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA,      \
-                        "%s failed: %s", #call, cudaGetErrorString(e_));                                  \
+        if (e_ != cudaSuccess) return fail(ctx, cvx_code(e_), "%s failed: %s", #call, cudaGetErrorString(e_)); \
     } while (0)
 
-int validate_setup(cvx_ctx* ctx, const cvx_frame_setup* s, int total) {
-    const int W = ctx->width, H = ctx->height;
+bool pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }
+
+// Raybuffer `which` (0 = top/down, 1 = left/right; RenderManager.cs:35-36): W + 2H rows of H pixels, or 2W + H rows of W pixels
+int raybuffer_rows(const cvx_ctx* ctx, int which) { return which == 0 ? ctx->width + 2 * ctx->height : 2 * ctx->width + ctx->height; }
+int raybuffer_row_length(const cvx_ctx* ctx, int which) { return which == 0 ? ctx->height : ctx->width; }
+int64_t raybuffer_pixels(const cvx_ctx* ctx, int which) { return (int64_t)raybuffer_rows(ctx, which) * raybuffer_row_length(ctx, which); }
+uint32_t* raybuffer(const cvx_slot& sl, int which) { return which == 0 ? sl.td : sl.lr; }
+
+cudaStream_t slot_stream(const cvx_ctx* ctx, int s) { return s == 0 ? ctx->stream : ctx->slots[s].stream; }
+
+int validate_setup(cvx_ctx* ctx, const cvx_frame_setup* s) {
     int tdRays = (s->segments[0].ray_count > 0 ? s->segments[0].ray_count : 0) + (s->segments[1].ray_count > 0 ? s->segments[1].ray_count : 0);
     int lrRays = (s->segments[2].ray_count > 0 ? s->segments[2].ray_count : 0) + (s->segments[3].ray_count > 0 ? s->segments[3].ray_count : 0);
-    if (tdRays > W + 2 * H || lrRays > 2 * W + H)
-        return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "segment ray counts (%d top/down, %d left/right) exceed the raybuffers (%d, %d rows)", tdRays, lrRays, W + 2 * H, 2 * W + H);
-    (void)total;
+    if (tdRays > raybuffer_rows(ctx, 0) || lrRays > raybuffer_rows(ctx, 1))
+        return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "segment ray counts (%d top/down, %d left/right) exceed the raybuffers (%d, %d rows)", tdRays, lrRays, raybuffer_rows(ctx, 0), raybuffer_rows(ctx, 1));
     // RenderManager.cs:482-483 clamps RayCount at 0; a negative count would give a negative row offset (host_frame.h: ray_index_offset)
     for (int k = 0; k < 4; k++)
         if (s->segments[k].ray_count < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "segment %d has a negative ray count (%d)", k, s->segments[k].ray_count);
     return CVX_OK;
 }
 
-void make_frame(cvx_ctx* ctx, const cvx_frame_setup* s, cvxd_frame& f) {
+// the frame of `s`, drawn into slot `slot`'s raybuffers
+void make_frame(cvx_ctx* ctx, const cvx_frame_setup* s, int slot, cvxd_frame& f) {
     cvxh::frame_from_setup(s, ctx->width, ctx->height, f);
     cvxd_frame_set_world(&f, &ctx->world); // also sets the distances of the last uploaded LOD and beyond to +inf
-    f.td = ctx->td; f.lr = ctx->lr;
+    f.td = ctx->slots[slot].td; f.lr = ctx->slots[slot].lr;
     f.counters = (ctx->flags & CVX_FLAG_COUNTERS) ? ctx->counters : nullptr;
     f.general_path = ctx->generalPath;
 }
 
-void make_blit(cvx_ctx* ctx, const cvxd_frame& f, uint32_t* target, cvxd_blit& b) {
+// Phase 2 of frame `f` into `target`: every row, from the raybuffers and rays of `f`
+void make_blit(const cvxd_frame& f, uint32_t* target, cvxd_blit& b) {
     memset(&b, 0, sizeof b);
     memcpy(b.seg, f.seg, sizeof b.seg);
     b.vp_x = f.vp_x; b.vp_y = f.vp_y;
-    b.width = ctx->width; b.height = ctx->height;
-    b.row_begin = 0; b.row_end = ctx->height;
-    b.ray_begin = 0; b.ray_end = f.total_rays; b.owned_only = 0;
-    b.td = ctx->td; b.lr = ctx->lr;
+    b.width = f.width; b.height = f.height;
+    b.row_begin = 0; b.row_end = f.height;
+    b.ray_begin = f.ray_begin; b.ray_end = f.ray_end; b.owned_only = 0;
+    b.il_chunk = f.il_chunk; b.il_ranks = f.il_ranks; b.il_rank = f.il_rank;
+    b.td = f.td; b.lr = f.lr;
     b.frame = target;
     cvxd_blit_prepare(&b);
+}
+
+// [begin, end) within [0, n): an end below 0 or past n means n
+void clamp_range(int& begin, int& end, int n) {
+    if (end < 0 || end > n) end = n;
+    if (begin < 0) begin = 0;
 }
 
 int check_ready(cvx_ctx* ctx, const void* setup) {
@@ -161,12 +178,31 @@ int check_ready(cvx_ctx* ctx, const void* setup) {
     return CVX_OK;
 }
 
-cudaStream_t slot_stream(cvx_ctx* ctx, int s) { return s == 0 ? ctx->stream : ctx->extra[s - 1].stream; }
-uint32_t* slot_td(cvx_ctx* ctx, int s) { return s == 0 ? ctx->td : ctx->extra[s - 1].td; }
-uint32_t* slot_lr(cvx_ctx* ctx, int s) { return s == 0 ? ctx->lr : ctx->extra[s - 1].lr; }
-uint32_t* slot_frame(cvx_ctx* ctx, int s) { return s == 0 ? ctx->frames[0] : ctx->extra[s - 1].frame; }
+// What the entry points that draw one setup start with: the context is ready and `f` is the frame of `setup` on slot `slot`,
+// checked against the raybuffers if `validate`, drawing the rays [ray_begin, ray_end) clamped to its rays
+int begin_frame(cvx_ctx* ctx, const cvx_frame_setup* setup, int slot, bool validate, int ray_begin, int ray_end, cvxd_frame& f) {
+    int r = check_ready(ctx, setup);
+    if (r) return r;
+    make_frame(ctx, setup, slot, f);
+    if (validate && (r = validate_setup(ctx, setup))) return r;
+    clamp_range(ray_begin, ray_end, f.total_rays);
+    f.ray_begin = ray_begin; f.ray_end = ray_end;
+    return CVX_OK;
+}
 
-uint32_t* current_target(cvx_ctx* ctx) { return ctx->externalFrame ? ctx->externalFrame : slot_frame(ctx, ctx->lastSlot); }
+// Event k of a view on `stream` (0: before Phase 1, 1: between the phases, 2: after Phase 2): cvx_last_draw_ms's events if `timed`,
+// and the view's cvx_profile_begin events while there is room for them
+cudaError_t mark_phase(cvx_ctx* ctx, int k, cudaStream_t stream, bool timed) {
+    cudaError_t e = cudaSuccess;
+    if (timed) e = cudaEventRecord(k == 0 ? ctx->evStart : k == 1 ? ctx->evMid : ctx->evEnd, stream);
+    if (e == cudaSuccess && timed && k == 2) ctx->timed = true;
+    const bool prof = ctx->profCount < ctx->profCapacity;
+    if (e == cudaSuccess && prof) e = cudaEventRecord(ctx->profEvents[3 * (size_t)ctx->profCount + k], stream);
+    if (e == cudaSuccess && prof && k == 2) ctx->profCount++;
+    return e;
+}
+
+uint32_t* current_target(cvx_ctx* ctx) { return ctx->externalFrame ? ctx->externalFrame : ctx->slots[ctx->lastSlot].frame; }
 
 // An asynchronous batch leaves its device->host copies unjoined (that is its point); its last view's frame lives in a slot's own
 // framebuffer until copied. Whatever else is about to WRITE a slot framebuffer first orders the context's stream behind those copies.
@@ -214,18 +250,26 @@ __global__ void ring_signal_kernel(uint32_t* flag, uint32_t value) {
 uint32_t* ring_frame(cvx_ctx* ctx, int slot) { return (uint32_t*)(ctx->ring + (size_t)slot * ctx->ringFrameBytes); }
 ring_flags* ring_flag_block(cvx_ctx* ctx, int slot) { return (ring_flags*)(ctx->ring + (size_t)ctx->ringSlots * ctx->ringFrameBytes) + slot; }
 
-void free_extra_slots(cvx_ctx* ctx) {
-    for (int i = 0; i < CVX_MAX_SLOTS - 1; i++) {
-        cvx_slot& sl = ctx->extra[i];
-        if (sl.stream) cudaStreamSynchronize(sl.stream);
-        cudaFree(sl.td); cudaFree(sl.lr); cudaFree(sl.frame);
-        sl.td = sl.lr = sl.frame = nullptr;
-    }
-    ctx->extraReady = 0;
-    ctx->lastSlot = 0;
-    if (ctx->copyStream) cudaStreamSynchronize(ctx->copyStream);
-    for (int i = 0; i < CVX_POOL_FRAMES; i++) { cudaFree(ctx->pool[i]); ctx->pool[i] = nullptr; ctx->poolUsed[i] = false; }
-    ctx->poolCount = 0;
+void free_slot(cvx_slot& sl) {
+    if (sl.stream) cudaStreamSynchronize(sl.stream);
+    cudaFree(sl.td); cudaFree(sl.lr); cudaFree(sl.frame);
+    sl.td = sl.lr = sl.frame = nullptr;
+}
+
+// zero-initialised raybuffers and framebuffer of the current resolution for slot s; nothing stays allocated if this fails
+cudaError_t alloc_slot(cvx_ctx* ctx, int s) {
+    cvx_slot& sl = ctx->slots[s];
+    const cudaStream_t stream = slot_stream(ctx, s);
+    const size_t tdBytes = (size_t)raybuffer_pixels(ctx, 0) * 4, lrBytes = (size_t)raybuffer_pixels(ctx, 1) * 4;
+    const size_t fbBytes = (size_t)ctx->width * ctx->height * 4;
+    cudaError_t e = cudaMalloc(&sl.td, tdBytes);
+    if (e == cudaSuccess) e = cudaMalloc(&sl.lr, lrBytes);
+    if (e == cudaSuccess) e = cudaMalloc(&sl.frame, fbBytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sl.td, 0, tdBytes, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sl.lr, 0, lrBytes, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sl.frame, 0, fbBytes, stream);
+    if (e != cudaSuccess) free_slot(sl);
+    return e;
 }
 
 // `want` pool framebuffers of the current resolution (events are created once per context)
@@ -238,50 +282,43 @@ int ensure_pool(cvx_ctx* ctx, int want) {
         if (!ctx->poolReady[i]) e = cudaEventCreateWithFlags(&ctx->poolReady[i], cudaEventDisableTiming);
         if (e == cudaSuccess && !ctx->poolFree[i]) e = cudaEventCreateWithFlags(&ctx->poolFree[i], cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaMalloc(&ctx->pool[i], fbBytes);
-        if (e != cudaSuccess) { ctx->pool[i] = nullptr; return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "frame pool allocation failed: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) { ctx->pool[i] = nullptr; return fail(ctx, cvx_code(e), "frame pool allocation failed: %s", cudaGetErrorString(e)); }
         ctx->poolCount++;
     }
     return CVX_OK;
 }
 
-// slots 1 .. want-1 get a stream, an event and zero-initialised buffers of the current resolution
+// slots 1 .. want-1 get a stream, an event and their buffers (slot 0 has its buffers from cvx_set_resolution)
 int ensure_slots(cvx_ctx* ctx, int want) {
     if (want > ctx->slotCount) want = ctx->slotCount;
-    const size_t W = (size_t)ctx->width, H = (size_t)ctx->height;
-    const size_t tdBytes = H * (W + 2 * H) * 4, lrBytes = W * (2 * W + H) * 4, fbBytes = W * H * 4;
-    while (ctx->extraReady < want - 1) {
-        cvx_slot& sl = ctx->extra[ctx->extraReady];
+    while (ctx->slotsReady < want) {
+        cvx_slot& sl = ctx->slots[ctx->slotsReady];
         cudaError_t e = cudaSuccess;
         if (!sl.stream) e = cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking);
         if (e == cudaSuccess && !sl.done) e = cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaMalloc(&sl.td, tdBytes);
-        if (e == cudaSuccess) e = cudaMalloc(&sl.lr, lrBytes);
-        if (e == cudaSuccess) e = cudaMalloc(&sl.frame, fbBytes);
-        if (e == cudaSuccess) e = cudaMemsetAsync(sl.td, 0, tdBytes, sl.stream);
-        if (e == cudaSuccess) e = cudaMemsetAsync(sl.lr, 0, lrBytes, sl.stream);
-        if (e == cudaSuccess) e = cudaMemsetAsync(sl.frame, 0, fbBytes, sl.stream);
-        if (e != cudaSuccess) {
-            cudaFree(sl.td); cudaFree(sl.lr); cudaFree(sl.frame);
-            sl.td = sl.lr = sl.frame = nullptr;
-            return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "frame slot allocation failed: %s", cudaGetErrorString(e));
-        }
-        ctx->extraReady++;
+        if (e == cudaSuccess) e = alloc_slot(ctx, ctx->slotsReady);
+        if (e != cudaSuccess) return fail(ctx, cvx_code(e), "frame slot allocation failed: %s", cudaGetErrorString(e));
+        ctx->slotsReady++;
     }
     return CVX_OK;
 }
 
+// everything sized by the resolution: the slots' buffers, the frame pool and the present staging frame
 void free_resolution(cvx_ctx* ctx) {
-    free_extra_slots(ctx);
-    cudaFree(ctx->td); cudaFree(ctx->lr); cudaFree(ctx->frames[0]); cudaFree(ctx->frames[1]); cudaFree(ctx->presentStage);
-    ctx->td = ctx->lr = ctx->frames[0] = ctx->frames[1] = ctx->presentStage = nullptr;
+    if (ctx->copyStream) cudaStreamSynchronize(ctx->copyStream);
+    for (cvx_slot& sl : ctx->slots) free_slot(sl);
+    ctx->slotsReady = 0;
+    ctx->lastSlot = 0;
+    for (int i = 0; i < CVX_POOL_FRAMES; i++) { cudaFree(ctx->pool[i]); ctx->pool[i] = nullptr; ctx->poolUsed[i] = false; }
+    ctx->poolCount = 0;
+    cudaFree(ctx->presentStage); ctx->presentStage = nullptr;
     ctx->width = ctx->height = 0;
 }
 
 void free_world(cvx_ctx* ctx) {
-    for (int i = 0; i < CVX_LOD_LEVELS; i++) {
-        cudaFree(ctx->lodHeaders[i]); cudaFree(ctx->lodElements[i]); cudaFree(ctx->lodBounds[i]);
-        ctx->lodHeaders[i] = ctx->lodElements[i] = ctx->lodBounds[i] = nullptr;
-        ctx->lodRegular[i] = false;
+    for (cvx_lod_memory& m : ctx->lod) {
+        cudaFree(m.headers); cudaFree(m.blob); cudaFree(m.bounds);
+        m = cvx_lod_memory();
     }
     memset(&ctx->world, 0, sizeof ctx->world);
 }
@@ -308,8 +345,9 @@ int install_lod(cvx_ctx* ctx, int lod, int dim_x, int dim_y, int dim_z, void* db
         return fail(ctx, r, "world upload failed: %s", err.c_str());
     }
     cudaStreamSynchronize(ctx->stream);
-    cudaFree(ctx->lodHeaders[lod]); cudaFree(ctx->lodElements[lod]); cudaFree(ctx->lodBounds[lod]);
-    ctx->lodHeaders[lod] = headers; ctx->lodElements[lod] = dblob; ctx->lodBounds[lod] = bounds;
+    cvx_lod_memory& m = ctx->lod[lod];
+    cudaFree(m.headers); cudaFree(m.blob); cudaFree(m.bounds);
+    m.blob = dblob; m.headers = headers; m.bounds = bounds; m.regular = regular != 0;
     cvxd_world_set_dims(&ctx->world, dim_x, dim_y, dim_z);
     cvxd_lod& l = ctx->world.lods[lod];
     l.headers = (const uint4*)headers;
@@ -317,9 +355,8 @@ int install_lod(cvx_ctx* ctx, int lod, int dim_x, int dim_y, int dim_z, void* db
     l.bounds = (const uint2*)bounds;
     l.mul_x = dim_z >> lod;
     l.lod = lod;
-    ctx->lodRegular[lod] = regular != 0;
     ctx->world.regular = 1;
-    for (int i = 0; i < CVX_LOD_LEVELS; i++) if (ctx->lodHeaders[i] && !ctx->lodRegular[i]) ctx->world.regular = 0;
+    for (const cvx_lod_memory& mi : ctx->lod) if (mi.headers && !mi.regular) ctx->world.regular = 0;
     if (lod + 1 > ctx->world.lod_count) ctx->world.lod_count = lod + 1;
     return CVX_OK;
 }
@@ -342,25 +379,22 @@ int cvx_create(const cvx_config* config, cvx_ctx** out_ctx) {
     ctx->device = dev;
     ctx->flags = config ? config->flags : 0;
     memset(&ctx->world, 0, sizeof ctx->world);
-    memset(ctx->lodHeaders, 0, sizeof ctx->lodHeaders);
-    memset(ctx->lodElements, 0, sizeof ctx->lodElements);
-    memset(ctx->lodBounds, 0, sizeof ctx->lodBounds);
-    memset(ctx->lodRegular, 0, sizeof ctx->lodRegular);
-#define CREATE_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail(nullptr, CVX_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); cvx_destroy(ctx); return CVX_ERR_CUDA; } } while (0)
-    CREATE_CU(cudaSetDevice(dev));
-    CREATE_CU(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-    CREATE_CU(cudaStreamCreateWithFlags(&ctx->copyStream, cudaStreamNonBlocking));
-    CREATE_CU(cudaEventCreate(&ctx->evStart));
-    CREATE_CU(cudaEventCreate(&ctx->evMid));
-    CREATE_CU(cudaEventCreate(&ctx->evEnd));
-    CREATE_CU(cudaEventCreateWithFlags(&ctx->evBatchStart, cudaEventDisableTiming));
-    for (int i = 0; i < 2; i++) {
-        CREATE_CU(cudaEventCreateWithFlags(&ctx->evFrameDone[i], cudaEventDisableTiming));
-        CREATE_CU(cudaEventCreateWithFlags(&ctx->evCopyDone[i], cudaEventDisableTiming));
-    }
-    CREATE_CU(cudaMalloc(&ctx->counters, sizeof(cvxd_counters)));
-    CREATE_CU(cudaMemset(ctx->counters, 0, sizeof(cvxd_counters)));
-#undef CREATE_CU
+    // without a context to hold it, a failure's message goes where cvx_last_error(NULL) finds it; the partial context is torn down
+    auto init = [ctx, dev]() -> int {
+        CU(nullptr, cudaSetDevice(dev));
+        CU(nullptr, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
+        CU(nullptr, cudaStreamCreateWithFlags(&ctx->copyStream, cudaStreamNonBlocking));
+        CU(nullptr, cudaEventCreate(&ctx->evStart));
+        CU(nullptr, cudaEventCreate(&ctx->evMid));
+        CU(nullptr, cudaEventCreate(&ctx->evEnd));
+        CU(nullptr, cudaEventCreateWithFlags(&ctx->evBatchStart, cudaEventDisableTiming));
+        CU(nullptr, cudaEventCreateWithFlags(&ctx->evFrameDone, cudaEventDisableTiming));
+        CU(nullptr, cudaEventCreateWithFlags(&ctx->evCopyDone, cudaEventDisableTiming));
+        CU(nullptr, cudaMalloc(&ctx->counters, sizeof(cvxd_counters)));
+        CU(nullptr, cudaMemset(ctx->counters, 0, sizeof(cvxd_counters)));
+        return CVX_OK;
+    };
+    if (int r = init()) { cvx_destroy(ctx); return r; }
     *out_ctx = ctx;
     return CVX_OK;
 }
@@ -377,17 +411,11 @@ int cvx_destroy(cvx_ctx* ctx) {
     for (cudaEvent_t e : ctx->profEvents) cudaEventDestroy(e);
     cvxjpeg::destroy(ctx->jpeg);
     cudaFree(ctx->counters);
-    if (ctx->evStart) cudaEventDestroy(ctx->evStart);
-    if (ctx->evMid) cudaEventDestroy(ctx->evMid);
-    if (ctx->evEnd) cudaEventDestroy(ctx->evEnd);
-    if (ctx->evBatchStart) cudaEventDestroy(ctx->evBatchStart);
-    for (int i = 0; i < CVX_MAX_SLOTS - 1; i++) {
-        if (ctx->extra[i].done) cudaEventDestroy(ctx->extra[i].done);
-        if (ctx->extra[i].stream) cudaStreamDestroy(ctx->extra[i].stream);
-    }
-    for (int i = 0; i < 2; i++) {
-        if (ctx->evFrameDone[i]) cudaEventDestroy(ctx->evFrameDone[i]);
-        if (ctx->evCopyDone[i]) cudaEventDestroy(ctx->evCopyDone[i]);
+    for (cudaEvent_t e : {ctx->evStart, ctx->evMid, ctx->evEnd, ctx->evBatchStart, ctx->evFrameDone, ctx->evCopyDone})
+        if (e) cudaEventDestroy(e);
+    for (cvx_slot& sl : ctx->slots) {
+        if (sl.done) cudaEventDestroy(sl.done);
+        if (sl.stream) cudaStreamDestroy(sl.stream);
     }
     for (int i = 0; i < 4; i++) if (ctx->batchDone[i]) cudaEventDestroy(ctx->batchDone[i]);
     for (int i = 0; i < CVX_POOL_FRAMES; i++) {
@@ -414,7 +442,6 @@ int cvx_set_stream(cvx_ctx* ctx, void* cuda_stream) {
 
 int cvx_world_upload(cvx_ctx* ctx, int32_t lod, int32_t dim_x, int32_t dim_y, int32_t dim_z, const void* blob, int64_t bytes, int32_t column_count) {
     if (!ctx) return CVX_ERR_INVALID_ARGUMENT;
-    auto pow2 = [](int n) { return n > 0 && (n & (n - 1)) == 0; };
     if (lod < 0 || lod >= CVX_LOD_LEVELS || !blob) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "bad lod %d or NULL blob", lod);
     if (!pow2(dim_x) || !pow2(dim_z) || dim_y < 1 || dim_y > 32768) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "world dimensions %dx%dx%d: x/z must be powers of two, y <= 32768", dim_x, dim_y, dim_z);
     const int64_t needCols = (int64_t)(dim_x >> lod) * (dim_z >> lod);
@@ -428,7 +455,7 @@ int cvx_world_upload(cvx_ctx* ctx, int32_t lod, int32_t dim_x, int32_t dim_y, in
     void* dblob = nullptr;
     cudaError_t e = cudaMalloc(&dblob, (size_t)(bytes > 0 ? bytes : 4));
     if (e == cudaSuccess) e = cudaMemcpyAsync(dblob, blob, (size_t)bytes, cudaMemcpyDefault, ctx->stream);
-    if (e != cudaSuccess) { cudaFree(dblob); return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "world upload failed: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { cudaFree(dblob); return fail(ctx, cvx_code(e), "world upload failed: %s", cudaGetErrorString(e)); }
     return install_lod(ctx, lod, dim_x, dim_y, dim_z, dblob, bytes, column_count);
 }
 
@@ -452,38 +479,26 @@ int cvx_set_resolution(cvx_ctx* ctx, int32_t width, int32_t height) {
     CU(ctx, cudaStreamSynchronize(ctx->copyStream));
     cvx_ring_close(ctx);  // its frames have the old size
     free_resolution(ctx);
-    const size_t tdBytes = (size_t)height * (size_t)(width + 2 * height) * 4; // RenderManager.cs:36
-    const size_t lrBytes = (size_t)width * (size_t)(2 * width + height) * 4;  // RenderManager.cs:35
-    const size_t fbBytes = (size_t)width * height * 4;
-    cudaError_t e = cudaMalloc(&ctx->td, tdBytes);
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->lr, lrBytes);
-    if (e == cudaSuccess) e = cudaMalloc(&ctx->frames[0], fbBytes);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->td, 0, tdBytes, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->lr, 0, lrBytes, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->frames[0], 0, fbBytes, ctx->stream);
+    ctx->width = width; ctx->height = height;
+    cudaError_t e = alloc_slot(ctx, 0);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) {
         free_resolution(ctx);
-        return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "raybuffer allocation failed: %s", cudaGetErrorString(e));
+        return fail(ctx, cvx_code(e), "raybuffer allocation failed: %s", cudaGetErrorString(e));
     }
-    ctx->width = width; ctx->height = height;
+    ctx->slotsReady = 1;
     return CVX_OK;
 }
 
 int cvx_draw_rays(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_begin, int32_t ray_end) {
-    int r = check_ready(ctx, setup);
-    if (r) return r;
     cvxd_frame f;
-    make_frame(ctx, setup, f);
-    if ((r = validate_setup(ctx, setup, f.total_rays))) return r;
-    if (ray_end < 0 || ray_end > f.total_rays) ray_end = f.total_rays;
-    if (ray_begin < 0) ray_begin = 0;
-    f.ray_begin = ray_begin; f.ray_end = ray_end;
+    int r = begin_frame(ctx, setup, 0, true, ray_begin, ray_end, f);
+    if (r) return r;
     ctx->lastSlot = 0;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaEventRecord(ctx->evStart, ctx->stream));
     CU(ctx, cvxd_launch_phase1(ctx->world, f, ctx->groupSize, ctx->stream));
-    if (ray_end > ray_begin) ctx->launches++;
+    if (f.ray_end > f.ray_begin) ctx->launches++;
     CU(ctx, cudaEventRecord(ctx->evMid, ctx->stream));
     CU(ctx, cudaEventRecord(ctx->evEnd, ctx->stream));
     ctx->timed = true;
@@ -491,14 +506,12 @@ int cvx_draw_rays(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_begin,
 }
 
 int cvx_blit_rows(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t row_begin, int32_t row_end) {
-    int r = check_ready(ctx, setup);
-    if (r) return r;
     cvxd_frame f;
-    make_frame(ctx, setup, f);
+    int r = begin_frame(ctx, setup, 0, false, 0, -1, f);
+    if (r) return r;
     cvxd_blit b;
-    make_blit(ctx, f, current_target(ctx), b);
-    if (row_end < 0 || row_end > ctx->height) row_end = ctx->height;
-    if (row_begin < 0) row_begin = 0;
+    make_blit(f, current_target(ctx), b);
+    clamp_range(row_begin, row_end, ctx->height);
     b.row_begin = row_begin; b.row_end = row_end;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, settle_async(ctx));
@@ -508,15 +521,12 @@ int cvx_blit_rows(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t row_begin,
 }
 
 int cvx_blit_owned(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_begin, int32_t ray_end, void* device_frame) {
-    int r = check_ready(ctx, setup);
-    if (r) return r;
     cvxd_frame f;
-    make_frame(ctx, setup, f);
+    int r = begin_frame(ctx, setup, 0, false, ray_begin, ray_end, f);
+    if (r) return r;
     cvxd_blit b;
-    make_blit(ctx, f, device_frame ? (uint32_t*)device_frame : current_target(ctx), b);
-    if (ray_end < 0 || ray_end > f.total_rays) ray_end = f.total_rays;
-    if (ray_begin < 0) ray_begin = 0;
-    b.ray_begin = ray_begin; b.ray_end = ray_end; b.owned_only = 1;
+    make_blit(f, device_frame ? (uint32_t*)device_frame : current_target(ctx), b);
+    b.owned_only = 1;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, settle_async(ctx));
     CU(ctx, cvxd_launch_phase2(b, ctx->stream));
@@ -526,35 +536,28 @@ int cvx_blit_owned(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_begin
 
 static int draw_into(cvx_ctx* ctx, const cvx_frame_setup* setup, int slot, uint32_t* target, bool timed) {
     cvxd_frame f;
+    int r;
     {
         CVX_RANGE("Segment setup overhead"); // RenderManager.cs:277: the SegmentContext fill
-        make_frame(ctx, setup, f);
+        r = begin_frame(ctx, setup, slot, true, 0, -1, f);
     }
-    f.td = slot_td(ctx, slot); f.lr = slot_lr(ctx, slot);
-    int r = validate_setup(ctx, setup, f.total_rays);
     if (r) return r;
     cvxd_blit b;
-    make_blit(ctx, f, target, b);
-    b.td = f.td; b.lr = f.lr;
+    make_blit(f, target, b);
     cudaStream_t stream = slot_stream(ctx, slot);
-    const bool prof = ctx->profCount < ctx->profCapacity;
-    cudaEvent_t* pe = prof ? &ctx->profEvents[3 * (size_t)ctx->profCount] : nullptr;
-    if (timed) CU(ctx, cudaEventRecord(ctx->evStart, stream));
-    if (prof) CU(ctx, cudaEventRecord(pe[0], stream));
+    CU(ctx, mark_phase(ctx, 0, stream, timed));
     {
         CVX_RANGE("Draw planes");            // RenderManager.cs:154
         CU(ctx, cvxd_launch_phase1(ctx->world, f, ctx->groupSize, stream));
     }
     if (f.total_rays > 0) ctx->launches++;
-    if (timed) CU(ctx, cudaEventRecord(ctx->evMid, stream));
-    if (prof) CU(ctx, cudaEventRecord(pe[1], stream));
+    CU(ctx, mark_phase(ctx, 1, stream, timed));
     {
         CVX_RANGE("Blit raybuffer");         // RenderManager.cs:178
         CU(ctx, cvxd_launch_phase2(b, stream));
     }
     ctx->launches++;
-    if (timed) { CU(ctx, cudaEventRecord(ctx->evEnd, stream)); ctx->timed = true; }
-    if (prof) { CU(ctx, cudaEventRecord(pe[2], stream)); ctx->profCount++; }
+    CU(ctx, mark_phase(ctx, 2, stream, timed));
     ctx->lastSlot = slot;
     return CVX_OK;
 }
@@ -586,7 +589,7 @@ static int draw_batch_impl(cvx_ctx* ctx, const cvx_frame_setup* setups, int32_t 
     // A caller-owned external frame forces one slot (one target buffer).
     const int K = ctx->externalFrame ? 1 : (ctx->slotCount < n_views ? ctx->slotCount : n_views);
     for (int i = 0; i < n_views; i++)  // every view is checked before the first one is enqueued
-        if ((r = validate_setup(ctx, setups + i, 0))) return r;
+        if ((r = validate_setup(ctx, setups + i))) return r;
     if ((r = ensure_slots(ctx, K))) return r;
     const bool pooled = dst_frames && !ctx->externalFrame && n_views > 1;
     const int M = CVX_POOL_FRAMES < n_views - 1 ? CVX_POOL_FRAMES : n_views - 1;
@@ -601,14 +604,14 @@ static int draw_batch_impl(cvx_ctx* ctx, const cvx_frame_setup* setups, int32_t 
         if (pooled) {
             const bool last = i == n_views - 1;
             const int pf = i % M;
-            uint32_t* target = last ? slot_frame(ctx, slot) : ctx->pool[pf];
+            uint32_t* target = last ? ctx->slots[slot].frame : ctx->pool[pf];
             // the previous user of the buffer (view i - M, or a view of an earlier asynchronous batch) has been copied out; the last view's
             // own framebuffer may still be read by the previous asynchronous batch's final copy
             if (!last && ctx->poolUsed[pf]) ce = cudaStreamWaitEvent(st, ctx->poolFree[pf], 0);
             if (last && ctx->batchSeq > 0) ce = cudaStreamWaitEvent(st, ctx->batchDone[(ctx->batchSeq - 1) % 4], 0);
             if (ce == cudaSuccess) r = draw_into(ctx, setups + i, slot, target, false);
             if (r || ce != cudaSuccess) break;
-            cudaEvent_t ready = last ? ctx->evFrameDone[0] : ctx->poolReady[pf];
+            cudaEvent_t ready = last ? ctx->evFrameDone : ctx->poolReady[pf];
             ce = cudaEventRecord(ready, st);
             if (ce == cudaSuccess) ce = cudaStreamWaitEvent(ctx->copyStream, ready, 0);
             // the copy is asynchronous only if dst_frames is page-locked (cvx_alloc_pinned / cudaHostRegister)
@@ -616,7 +619,7 @@ static int draw_batch_impl(cvx_ctx* ctx, const cvx_frame_setup* setups, int32_t 
             if (ce == cudaSuccess && !last) { ce = cudaEventRecord(ctx->poolFree[pf], ctx->copyStream); ctx->poolUsed[pf] = true; }
             continue;
         }
-        uint32_t* target = ctx->externalFrame ? ctx->externalFrame : slot_frame(ctx, slot);
+        uint32_t* target = ctx->externalFrame ? ctx->externalFrame : ctx->slots[slot].frame;
         r = draw_into(ctx, setups + i, slot, target, false);
         if (!r && dst_frames) ce = cudaMemcpyAsync((uint8_t*)dst_frames + (size_t)i * fbBytes, target, fbBytes, cudaMemcpyDeviceToHost, st);
     }
@@ -627,15 +630,15 @@ static int draw_batch_impl(cvx_ctx* ctx, const cvx_frame_setup* setups, int32_t 
         }
         if (ce == cudaSuccess) ce = cudaEventRecord(ctx->batchDone[ctx->batchSeq % 4], ctx->copyStream);
     } else if (pooled) {     // the context's stream also waits for the copies
-        cudaError_t e1 = cudaEventRecord(ctx->evCopyDone[0], ctx->copyStream);
-        if (e1 == cudaSuccess) e1 = cudaStreamWaitEvent(ctx->stream, ctx->evCopyDone[0], 0);
+        cudaError_t e1 = cudaEventRecord(ctx->evCopyDone, ctx->copyStream);
+        if (e1 == cudaSuccess) e1 = cudaStreamWaitEvent(ctx->stream, ctx->evCopyDone, 0);
         if (ce == cudaSuccess) ce = e1;
     }
     // join — also after a failure in the middle of the batch, so that the slots' work stays ordered before whatever the caller
     // queues next on the context's stream (events, reads, the next batch)
     for (int s = 1; s < K; s++) {
-        cudaError_t e1 = cudaEventRecord(ctx->extra[s - 1].done, slot_stream(ctx, s));
-        if (e1 == cudaSuccess) e1 = cudaStreamWaitEvent(ctx->stream, ctx->extra[s - 1].done, 0);
+        cudaError_t e1 = cudaEventRecord(ctx->slots[s].done, ctx->slots[s].stream);
+        if (e1 == cudaSuccess) e1 = cudaStreamWaitEvent(ctx->stream, ctx->slots[s].done, 0);
         if (ce == cudaSuccess) ce = e1;
     }
     if (r) return r;
@@ -705,7 +708,7 @@ int cvx_sync(cvx_ctx* ctx) {
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->copyStream));
     if (ctx->ring)  // sharded views run on the slot streams without a join into the context's stream
-        for (int i = 0; i < CVX_MAX_SLOTS - 1; i++) if (ctx->extra[i].stream) CU(ctx, cudaStreamSynchronize(ctx->extra[i].stream));
+        for (const cvx_slot& sl : ctx->slots) if (sl.stream) CU(ctx, cudaStreamSynchronize(sl.stream));
     return CVX_OK;
 }
 
@@ -717,8 +720,8 @@ int cvx_blit_raybuffer(cvx_ctx* ctx, int32_t which) {
     const int W = ctx->width, H = ctx->height;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, settle_async(ctx));
-    const uint32_t* buf = which == 0 ? slot_td(ctx, ctx->lastSlot) : slot_lr(ctx, ctx->lastSlot);
-    CU(ctx, cvxd_launch_raybuffer_view(buf, which == 0 ? W + 2 * H : 2 * W + H, which == 0 ? H : W, current_target(ctx), W, H, ctx->stream));
+    const uint32_t* buf = raybuffer(ctx->slots[ctx->lastSlot], which);
+    CU(ctx, cvxd_launch_raybuffer_view(buf, raybuffer_rows(ctx, which), raybuffer_row_length(ctx, which), current_target(ctx), W, H, ctx->stream));
     ctx->launches++;
     return CVX_OK;
 }
@@ -737,7 +740,7 @@ int cvx_present(cvx_ctx* ctx, int32_t format, int32_t top_down, void* dst, int32
     if (!dst_is_device) {
         if (!ctx->presentStage) {
             cudaError_t e = cudaMalloc(&ctx->presentStage, fbBytes);
-            if (e != cudaSuccess) return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "present staging allocation failed: %s", cudaGetErrorString(e));
+            if (e != cudaSuccess) return fail(ctx, cvx_code(e), "present staging allocation failed: %s", cudaGetErrorString(e));
         }
         out = ctx->presentStage;
     }
@@ -770,7 +773,7 @@ int cvx_present_jpeg(cvx_ctx* ctx, int32_t quality, int32_t subsampling, void* d
     }
     if (!ctx->presentStage) {
         cudaError_t e = cudaMalloc(&ctx->presentStage, (size_t)W * H * 4);
-        if (e != cudaSuccess) return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "present staging allocation failed: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, cvx_code(e), "present staging allocation failed: %s", cudaGetErrorString(e));
     }
     CU(ctx, cvxd_launch_present_rgb8(current_target(ctx), (uint8_t*)ctx->presentStage, W, H, 1, ctx->stream));
     ctx->launches++;
@@ -819,7 +822,6 @@ int cvx_world_build_from_mesh(cvx_ctx* ctx, const float* positions, const uint8_
     int dims[3];
     int r = cvxh_remap_mesh(positions, n_vertices, max_dimension, flips, xyz, dims);
     if (r) return fail(ctx, r, "mesh cannot be remapped to max dimension %d", max_dimension);
-    auto pow2 = [](int n) { return n > 0 && (n & (n - 1)) == 0; };
     if (!pow2(dims[0]) || !pow2(dims[2])) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "world dimensions %dx%dx%d: x/z must be powers of two", dims[0], dims[1], dims[2]);
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
@@ -849,7 +851,7 @@ int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_r
     if (n > 0 && (!rays || !out)) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "rays or hits is NULL");
     if (n == 0) return CVX_OK;
     CU(ctx, cudaSetDevice(ctx->device));
-    const bool bounds = ctx->lodRegular[lod] && !ctx->generalPath;
+    const bool bounds = ctx->lod[lod].regular && !ctx->generalPath;
     if (on_device) {
         CU(ctx, cvxd_launch_raycast(ctx->world, lod, (const cvxd_ray*)rays, (cvxd_ray_hit*)out, n, bounds, ctx->stream));
         ctx->launches++;
@@ -860,7 +862,7 @@ int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_r
         CU(ctx, cudaStreamSynchronize(ctx->stream));
         free_ray_scratch(ctx);
         cudaError_t e = cudaMalloc(&ctx->rayScratch, need);
-        if (e != cudaSuccess) { ctx->rayScratch = nullptr; return fail(ctx, e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA, "ray scratch allocation failed: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) { ctx->rayScratch = nullptr; return fail(ctx, cvx_code(e), "ray scratch allocation failed: %s", cudaGetErrorString(e)); }
         ctx->rayScratchBytes = need;
     }
     cvxd_ray* dRays = (cvxd_ray*)ctx->rayScratch;
@@ -887,11 +889,10 @@ int cvx_read_frame(cvx_ctx* ctx, void* dst_argb, int64_t bytes) {
 int cvx_read_raybuffer(cvx_ctx* ctx, int32_t which, void* dst_argb, int64_t bytes) {
     if (!ctx || !dst_argb || which < 0 || which > 1) return CVX_ERR_INVALID_ARGUMENT;
     if (ctx->width <= 0) return fail(ctx, CVX_ERR_NO_RESOLUTION, "no resolution set");
-    const int64_t W = ctx->width, H = ctx->height;
-    const int64_t full = which == 0 ? H * (W + 2 * H) * 4 : W * (2 * W + H) * 4;
+    const int64_t full = raybuffer_pixels(ctx, which) * 4;
     const int64_t n = bytes < full ? bytes : full;
     CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, cudaMemcpyAsync(dst_argb, which == 0 ? slot_td(ctx, ctx->lastSlot) : slot_lr(ctx, ctx->lastSlot), (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(dst_argb, raybuffer(ctx->slots[ctx->lastSlot], which), (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return CVX_OK;
 }
@@ -899,10 +900,9 @@ int cvx_read_raybuffer(cvx_ctx* ctx, int32_t which, void* dst_argb, int64_t byte
 int cvx_clear_raybuffers(cvx_ctx* ctx, uint32_t argb) { // RenderManager.ClearRayBuffer (debug), RenderManager.cs:58-92
     if (!ctx) return CVX_ERR_INVALID_ARGUMENT;
     if (ctx->width <= 0) return fail(ctx, CVX_ERR_NO_RESOLUTION, "no resolution set");
-    const int64_t W = ctx->width, H = ctx->height;
     CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, cvxd_launch_fill(ctx->td, argb, H * (W + 2 * H), ctx->stream));
-    CU(ctx, cvxd_launch_fill(ctx->lr, argb, W * (2 * W + H), ctx->stream));
+    CU(ctx, cvxd_launch_fill(ctx->slots[0].td, argb, raybuffer_pixels(ctx, 0), ctx->stream));
+    CU(ctx, cvxd_launch_fill(ctx->slots[0].lr, argb, raybuffer_pixels(ctx, 1), ctx->stream));
     ctx->launches += 2;
     return CVX_OK;
 }
@@ -927,9 +927,8 @@ int cvx_device_frame(cvx_ctx* ctx, void** out_device_ptr, int64_t* out_bytes) {
 int cvx_device_raybuffer(cvx_ctx* ctx, int32_t which, void** out_device_ptr, int64_t* out_bytes) {
     if (!ctx || !out_device_ptr || which < 0 || which > 1) return CVX_ERR_INVALID_ARGUMENT;
     if (ctx->width <= 0) return fail(ctx, CVX_ERR_NO_RESOLUTION, "no resolution set");
-    const int64_t W = ctx->width, H = ctx->height;
-    *out_device_ptr = which == 0 ? slot_td(ctx, ctx->lastSlot) : slot_lr(ctx, ctx->lastSlot);
-    if (out_bytes) *out_bytes = which == 0 ? H * (W + 2 * H) * 4 : W * (2 * W + H) * 4;
+    *out_device_ptr = raybuffer(ctx->slots[ctx->lastSlot], which);
+    if (out_bytes) *out_bytes = raybuffer_pixels(ctx, which) * 4;
     return CVX_OK;
 }
 
@@ -1020,11 +1019,10 @@ int cvx_profile_end(cvx_ctx* ctx, double* out_phase1_ms, double* out_phase2_ms, 
 }
 
 int cvx_debug_ray_setup(cvx_ctx* ctx, const cvx_frame_setup* setup, cvx_ray_state* out, int32_t max_rays) {
-    int r = check_ready(ctx, setup);
+    cvxd_frame f;
+    int r = begin_frame(ctx, setup, 0, false, 0, -1, f);
     if (r) return r;
     if (!out || max_rays < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "bad output buffer");
-    cvxd_frame f;
-    make_frame(ctx, setup, f);
     int n = f.total_rays < max_rays ? f.total_rays : max_rays;
     if (n == 0) return f.total_rays;
     CU(ctx, cudaSetDevice(ctx->device));
@@ -1040,12 +1038,11 @@ int cvx_debug_ray_setup(cvx_ctx* ctx, const cvx_frame_setup* setup, cvx_ray_stat
 }
 
 int cvx_debug_ray_timing(cvx_ctx* ctx, const cvx_frame_setup* setup, int64_t* out_cycles, int32_t max_rays) {
-    int r = check_ready(ctx, setup);
+    cvxd_frame f;
+    int r = begin_frame(ctx, setup, 0, false, 0, -1, f);
     if (r) return r;
     if (!out_cycles || max_rays < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "bad output buffer");
-    cvxd_frame f;
-    make_frame(ctx, setup, f);
-    if ((r = validate_setup(ctx, setup, f.total_rays))) return r;
+    if ((r = validate_setup(ctx, setup))) return r;
     const int n = f.total_rays < max_rays ? f.total_rays : max_rays;
     if (n == 0) return f.total_rays;
     CU(ctx, cudaSetDevice(ctx->device));
@@ -1069,7 +1066,7 @@ int cvx_ipc_export_frame(cvx_ctx* ctx, uint8_t out_handle[CVX_IPC_HANDLE_BYTES])
     if (ctx->width <= 0) return fail(ctx, CVX_ERR_NO_RESOLUTION, "no resolution set");
     CU(ctx, cudaSetDevice(ctx->device));
     cudaIpcMemHandle_t h;
-    CU(ctx, cudaIpcGetMemHandle(&h, ctx->frames[0]));
+    CU(ctx, cudaIpcGetMemHandle(&h, ctx->slots[0].frame));
     memcpy(out_handle, &h, sizeof h);
     return CVX_OK;
 }
@@ -1100,7 +1097,7 @@ int cvx_ring_close(cvx_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     cudaStreamSynchronize(ctx->copyStream);
-    for (int i = 0; i < CVX_MAX_SLOTS - 1; i++) if (ctx->extra[i].stream) cudaStreamSynchronize(ctx->extra[i].stream);
+    for (const cvx_slot& sl : ctx->slots) if (sl.stream) cudaStreamSynchronize(sl.stream);
     if (ctx->ringOwner) cudaFree(ctx->ring); else cudaIpcCloseMemHandle(ctx->ring);
     ctx->ring = nullptr; ctx->ringSlots = 0; ctx->ringWorld = 0; ctx->ringOwner = false;
     return CVX_OK;
@@ -1148,17 +1145,15 @@ int cvx_draw_sharded(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_beg
     if (r) return r;
     if (!ctx->ring) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "no frame ring (cvx_ring_create / cvx_ring_open)");
     if (rank < 0 || rank >= ctx->ringWorld || view_index < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "rank %d / view %lld outside the ring", rank, (long long)view_index);
-    if ((r = validate_setup(ctx, setup, 0))) return r;
+    if ((r = validate_setup(ctx, setup))) return r;
     CU(ctx, cudaSetDevice(ctx->device));
     const int K = ctx->slotCount;
     if ((r = ensure_slots(ctx, K))) return r;
     const int slot = (int)(view_index % K), rslot = (int)(view_index % ctx->ringSlots);
     cudaStream_t stream = slot_stream(ctx, slot);
     cvxd_frame f;
-    make_frame(ctx, setup, f);
-    f.td = slot_td(ctx, slot); f.lr = slot_lr(ctx, slot);
-    const bool interleaved = ray_begin == CVX_SHARD_INTERLEAVED;
-    if (interleaved) {
+    make_frame(ctx, setup, slot, f);
+    if (ray_begin == CVX_SHARD_INTERLEAVED) {
         // rays dealt in chunks of `ray_end` rays, chunk c to rank c mod world: heavy rays come in runs of neighbouring rays, so every
         // rank gets its share of them without any cost estimate; the launch covers the rank's local rays [0, n)
         const int chunk = ray_end;
@@ -1171,14 +1166,11 @@ int cvx_draw_sharded(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_beg
         f.il_chunk = chunk; f.il_ranks = world; f.il_rank = rank;
         ray_begin = 0; ray_end = n;
     } else {
-        if (ray_end < 0 || ray_end > f.total_rays) ray_end = f.total_rays;
-        if (ray_begin < 0) ray_begin = 0;
+        clamp_range(ray_begin, ray_end, f.total_rays);
     }
     f.ray_begin = ray_begin; f.ray_end = ray_end;
     ring_flags* fl = ring_flag_block(ctx, rslot);
-    const bool prof = ctx->profCount < ctx->profCapacity;   // cvx_profile_begin: events around this share's Phase 1 and Phase 2
-    cudaEvent_t* pe = prof ? &ctx->profEvents[3 * (size_t)ctx->profCount] : nullptr;
-    if (prof) CU(ctx, cudaEventRecord(pe[0], stream));
+    CU(ctx, mark_phase(ctx, 0, stream, false));   // cvx_profile_begin: events around this share's Phase 1 and Phase 2
     CU(ctx, cvxd_launch_phase1(ctx->world, f, ctx->groupSize, stream));   // Phase 1 writes this rank's own raybuffers: no need to wait for the ring
     if (ray_end > ray_begin) ctx->launches++;
     if (view_index >= ctx->ringSlots) {  // the ring frame still holds view_index - slots until the root releases it
@@ -1186,13 +1178,11 @@ int cvx_draw_sharded(cvx_ctx* ctx, const cvx_frame_setup* setup, int32_t ray_beg
         ctx->launches++;
     }
     cvxd_blit b;
-    make_blit(ctx, f, ring_frame(ctx, rslot), b);
-    b.td = f.td; b.lr = f.lr;
-    b.ray_begin = ray_begin; b.ray_end = ray_end; b.owned_only = 1;
-    b.il_chunk = f.il_chunk; b.il_ranks = f.il_ranks; b.il_rank = f.il_rank;
-    if (prof) CU(ctx, cudaEventRecord(pe[1], stream));
+    make_blit(f, ring_frame(ctx, rslot), b);
+    b.owned_only = 1;
+    CU(ctx, mark_phase(ctx, 1, stream, false));
     CU(ctx, cvxd_launch_phase2(b, stream));
-    if (prof) { CU(ctx, cudaEventRecord(pe[2], stream)); ctx->profCount++; }
+    CU(ctx, mark_phase(ctx, 2, stream, false));
     ring_signal_kernel<<<1, 1, 0, stream>>>(&fl->arrive[rank], (uint32_t)(view_index + 1));
     ctx->launches += 2;
     CU(ctx, cudaGetLastError());
@@ -1231,7 +1221,7 @@ int cvx_ring_status(cvx_ctx* ctx) {
 int cvx_alloc_pinned(int64_t bytes, void** out) {
     if (!out || bytes <= 0) return CVX_ERR_INVALID_ARGUMENT;
     cudaError_t e = cudaHostAlloc(out, (size_t)bytes, cudaHostAllocDefault);
-    return e == cudaSuccess ? CVX_OK : (e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA);
+    return e == cudaSuccess ? CVX_OK : cvx_code(e);
 }
 
 int cvx_free_pinned(void* p) { return cudaFreeHost(p) == cudaSuccess ? CVX_OK : CVX_ERR_CUDA; }

@@ -43,6 +43,8 @@ int cvxh_remap_mesh(const float* positions, int32_t n_vertices, int32_t max_dime
 #ifdef __CUDACC__
 #include <functional>
 #include <string>
+/* The CVX_ERR_* code a failed CUDA call reports: running out of device memory is told apart from every other failure. */
+inline int cvx_code(cudaError_t e) { return e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA; }
 /* Receives each finished LOD blob while it is still in device memory and takes ownership of the allocation (cudaFree it). */
 typedef std::function<int(int lod, void* device_blob, int64_t bytes, int column_count)> cvxd_lod_sink;
 /* world_builder_gpu.cu: voxelize + RLE + LOD mips on the device (b->dims set by the caller). Without a sink the blobs are copied into

@@ -228,7 +228,7 @@ struct DeviceBuffers {
     void release(void* p) { for (auto& q : all) if (q == p) { cudaFree(p); q = nullptr; } }
 };
 
-#define CK(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { err = std::string(#expr) + ": " + cudaGetErrorString(e_); return e_ == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA; } } while (0)
+#define CK(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { err = std::string(#expr) + ": " + cudaGetErrorString(e_); return cvx_code(e_); } } while (0)
 
 inline int bits_for(unsigned long long maxKey) { int b = 1; while (b < 64 && (maxKey >> b) != 0ull) b++; return b; }
 
@@ -402,7 +402,7 @@ int cvxd_transcode_lod_device(cudaStream_t stream, const void* blob_dev, int64_t
     void* headers = nullptr; void* bounds = nullptr;
     CK(cudaMalloc(&headers, (size_t)(16 * need_cols)));
     cudaError_t e = cudaMalloc(&bounds, total ? (size_t)total * 8 : 8);
-    if (e != cudaSuccess) { cudaFree(headers); err = cudaGetErrorString(e); return e == cudaErrorMemoryAllocation ? CVX_ERR_OUT_OF_MEMORY : CVX_ERR_CUDA; }
+    if (e != cudaSuccess) { cudaFree(headers); err = cudaGetErrorString(e); return cvx_code(e); }
     transcode_write_kernel<<<blocks, 256, 0, stream>>>(words, elements, need_cols, lod, dim_y, offsets, (uint4*)headers, (uint2*)bounds, irregular);
     int hostIrregular = 1;
     e = cudaGetLastError();
