@@ -281,13 +281,43 @@ __device__ __forceinline__ int mark_seen(uint32_t* seen, int a, int b, int gl) {
     return fresh;
 }
 
+// Per-ray state that is the same in every lane of the group and that the column loops read rarely: the DDA state between batches
+// (read and advanced once per batch), the projected plane of the ray (read once per round and once per re-narrowing), the raybuffer
+// row and the original writable range (read once per committed span). It lives in shared memory, one copy per group, instead of one
+// register copy per lane; the registers go to more resident warps (DESIGN.md §7.1).
+struct P1Group {
+    Dda ray;                            // the cell after the last batch
+    F3 planeBottom, planeTop, planeDir; // SetupProjectedPlaneParams :622-651
+    uint32_t* row;                      // raybuffer row
+    int orig_min, orig_max;             // originalNextFreePixelMin/Max
+};
+
+// Dynamic shared memory of a Phase-1 CTA: the P1Group of each group, then per group the written-pixel mask (one word per 32 pixels of
+// the longest row), G ints (lane of a round -> batch cell of its column) and the 7 x G words of the round cache.
+static size_t phase1_smem_bytes(int G, int width, int height) {
+    const int seenWords = ((width > height ? width : height) + 31) >> 5;
+    return (size_t)(CVXD_THREADS_PER_CTA / G) * (sizeof(P1Group) + (size_t)(seenWords + 8 * G) * sizeof(uint32_t));
+}
+
 struct RowState {
     uint32_t* seen;         // shared-memory bitmask of this row
-    uint32_t* row;          // raybuffer row
-    int orig_min, orig_max; // originalNextFreePixelMin/Max
+    const P1Group* grp;     // raybuffer row and original writable range
     int nf_min, nf_max;     // nextFreePixelMin/Max
     float fb_min, fb_max;   // frustumBoundsMin/Max
 };
+
+// RLEElement (World.cs:245-259) as one word: colour index in the low half, length in the high half, both signed 16-bit
+__device__ __forceinline__ int el_ci(uint32_t e) { return (int)(short)(e & 0xffffu); }
+__device__ __forceinline__ int el_len(uint32_t e) { return (int)(short)(e >> 16); }
+// A pixel span [lo, hi] of the round cache as one word: two signed 16-bit halves, each end saturated to 16 bits. Pixel indices lie below
+// CVXD_MAX_AXIS, so a saturated end falls on the same side of nextFreePixelMin/Max as the true one: span_would_write answers the same,
+// and reduce_pixel_horizon clamps it to the same pixel or moves nextFreePixelMin/Max past the other end either way (the ray then ends).
+__device__ __forceinline__ uint32_t span_pack(int lo, int hi) {
+    lo = max(-32768, min(32767, lo)); hi = max(-32768, min(32767, hi));
+    return ((uint32_t)lo & 0xffffu) | ((uint32_t)hi << 16);
+}
+__device__ __forceinline__ int span_lo(uint32_t s) { return (int)(short)(s & 0xffffu); }
+__device__ __forceinline__ int span_hi(uint32_t s) { return (int)s >> 16; }
 
 // A span [bMin, bMax] changes anything (pixels, horizon, frustum) only if it holds a still-unwritten pixel of the
 // writable range: nextFreePixelMin/Max are themselves unwritten pixels (the scans of :407-415,678-692 stop on one),
@@ -304,14 +334,14 @@ __device__ __forceinline__ void reduce_pixel_horizon(RowState& rw, int& bMin, in
     if (bMin <= rw.nf_min) {
         bMin = rw.nf_min;
         if (bMax >= rw.nf_min) {
-            rw.nf_min = scan_up(rw.seen, bMax + 1, rw.orig_max);
+            rw.nf_min = scan_up(rw.seen, bMax + 1, rw.grp->orig_max);
             rw.fb_min = rw.nf_min - 0.501f;
         }
     }
     if (bMax >= rw.nf_max) {
         bMax = rw.nf_max;
         if (bMin <= rw.nf_max) {
-            rw.nf_max = scan_down(rw.seen, bMin - 1, rw.orig_min);
+            rw.nf_max = scan_down(rw.seen, bMin - 1, rw.grp->orig_min);
             rw.fb_max = rw.nf_max + 0.501f;
         }
     }
@@ -324,8 +354,8 @@ struct Acc { unsigned long long dda_steps, columns_nonempty, runs_visited, px_vo
  * Neighbouring rows (adjacent rays of one segment) share a warp: they walk nearly the same columns, so the groups of
  * a warp stay mostly convergent while the number of rays in flight per SM grows by 32/G.
  */
-#ifndef CVXD_MIN_CTAS_PER_SM /* with 32-thread CTAs: 21 -> ptxas settles on 80 registers (25 resident warps per SM); measured best */
-#define CVXD_MIN_CTAS_PER_SM 21
+#ifndef CVXD_MIN_CTAS_PER_SM /* with 32-thread CTAs: 32 -> 64 registers, 32 resident warps per SM (profiles/r03_phase1_regs.md); measured best */
+#define CVXD_MIN_CTAS_PER_SM 32
 #endif
 #if CVXD_MIN_CTAS_PER_SM > 0
 #define CVXD_P1_BOUNDS __launch_bounds__(CVXD_THREADS_PER_CTA, CVXD_MIN_CTAS_PER_SM)
@@ -336,9 +366,9 @@ template <int G, bool COUNTERS, bool TIMING, bool FAST, bool INV>
 __global__ void CVXD_P1_BOUNDS
 phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ cvxd_frame f) {
 #ifdef CVX_EMU
-    uint32_t* seen_all = emu::g_shared;
+    uint32_t* smem_all = emu::g_shared;
 #else
-    extern __shared__ uint32_t seen_all[];
+    extern __shared__ __align__(16) uint32_t smem_all[]; // phase1_smem_bytes
 #endif
     constexpr int GROUPS_PER_CTA = CVXD_THREADS_PER_CTA / G;
     constexpr uint32_t GBITS = G == 32 ? FULL_MASK : ((1u << (G & 31)) - 1u);
@@ -372,47 +402,45 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
 
     Acc acc = {0, 0, 0, 0, 0}; // per lane; summed with atomics at the end (COUNTERS only)
     if (COUNTERS && gl == 0) acc.dda_steps = (unsigned long long)rs.lod_steps;
+    P1Group& gs = reinterpret_cast<P1Group*>(smem_all)[group]; // written by every lane with the same values
     RowState rw;
-    rw.seen = seen_all + group * (seenWords + 9 * G);
+    rw.seen = reinterpret_cast<uint32_t*>(reinterpret_cast<P1Group*>(smem_all) + GROUPS_PER_CTA) + group * (seenWords + 8 * G);
+    rw.grp = &gs;
     int* scratch = (int*)(rw.seen + seenWords); // G ints: lane of a round -> batch cell of its column
-    uint32_t* cache = (uint32_t*)(scratch + G); // 8 x G words: commit-only fields of the round cache
-    rw.row = row;
-    rw.orig_min = sg.pix_min; rw.orig_max = sg.pix_max;
-    rw.nf_min = rw.orig_min; rw.nf_max = rw.orig_max;
+    uint32_t* cache = (uint32_t*)(scratch + G); // 7 x G words: commit-only fields of the round cache
+    const int origMin = sg.pix_min, origMax = sg.pix_max;
+    rw.nf_min = origMin; rw.nf_max = origMax;
     rw.fb_min = rw.nf_min - 0.501f; rw.fb_max = rw.nf_max + 0.501f;
 
     if (rs.status == 1) { // WriteSkyboxFull :710-716
-        for (int y = rw.orig_min + gl; y <= rw.orig_max; y += G) row[y] = SKYBOX_ARGB;
-        if (COUNTERS && gl == 0 && rw.orig_max >= rw.orig_min) acc.px_sky += rw.orig_max - rw.orig_min + 1;
+        for (int y = origMin + gl; y <= origMax; y += G) row[y] = SKYBOX_ARGB;
+        if (COUNTERS && gl == 0 && origMax >= origMin) acc.px_sky += origMax - origMin + 1;
     } else {
         for (int w = gl; w < seenWords; w += G) rw.seen[w] = 0u; // stackalloc, zero-initialised (:208)
-        __syncwarp(gmask);
+        gs.ray = rs.dda;
+        gs.row = row;
+        gs.orig_min = origMin; gs.orig_max = origMax;
 
-        Dda ray = rs.dda;
         int lod = rs.lod;
-        int voxelScale = 1 << lod;
-        const float farClip = f.far_clip;
-        float lodMax = f.lod_dist[lod];
-        #define worldMaxY (world.dim_y_f) /* a constant-bank operand, not a register */
-        const float camY = f.pos_y;
+        #define worldMaxY (world.dim_y_f) /* constant-bank operands, not registers */
+        #define farClip (f.far_clip)
+        #define camY (f.pos_y)
         #define cameraPosYNormalized (f.cam_y_norm)
         constexpr int ITER = INV ? -1 : 1; // RenderJob.Execute :174-178 (INV = InverseElementIterationDirection, one kernel instance per direction)
         const float EPS = float_epsilon();
         float frustumDirMaxWorld = EPS, frustumDirMinWorld = EPS;
 
-        // SetupProjectedPlaneParams :622-651
-        F3 planeBottom, planeTop, planeDir;
-        {
+        { // SetupProjectedPlaneParams :622-651
             float top[4], bot[4], dir[4];
-            project(f.wts, ray.start_x, worldMaxY, ray.start_z, 1.0f, top);
-            project(f.wts, ray.start_x, 0.0f, ray.start_z, 1.0f, bot);
-            project(f.wts, ray.dir_x, 0.0f, ray.dir_z, 0.0f, dir);
-            const int a = sg.axis_mapped_to_y ? 1 : 0;
-            planeBottom = F3{bot[a], bot[2], bot[3]};
-            planeTop = F3{top[a], top[2], top[3]};
-            planeDir = F3{dir[a], dir[2], dir[3]};
+            project(f.wts, rs.dda.start_x, worldMaxY, rs.dda.start_z, 1.0f, top);
+            project(f.wts, rs.dda.start_x, 0.0f, rs.dda.start_z, 1.0f, bot);
+            project(f.wts, rs.dda.dir_x, 0.0f, rs.dda.dir_z, 0.0f, dir);
+            const bool a = sg.axis_mapped_to_y; // selected, not indexed: a computed index would put the arrays in local memory
+            gs.planeBottom = F3{a ? bot[1] : bot[0], bot[2], bot[3]};
+            gs.planeTop = F3{a ? top[1] : top[0], top[2], top[3]};
+            gs.planeDir = F3{a ? dir[1] : dir[0], dir[2], dir[3]};
         }
-        const int maskX = world.dim_x - 1, maskZ = world.dim_z - 1;
+        __syncwarp(gmask);
         // unlerp(0, worldMaxY, y) = (y - 0) / (worldMaxY - 0): for a power-of-two height the quotient is exactly y * 2^-k
 
         bool terminated = false; // ray ended inside the loop: skybox the rest and stop
@@ -429,11 +457,12 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
             // :237-243, tested once per visited cell: here for cell 0, for later cells by cutting the batch. This needs no LOD bound:
             // lod_dist of the last uploaded LOD is +inf (cvxd_frame_set_world), and dl is never +inf here, since every dl is a finite
             // crossing distance, a still axis contributes -inf (dda_step_to_world, dda_next_lod) and a NaN compares false.
-            if (ray.dl >= lodMax) {
-                dda_next_lod(ray, voxelScale);
-                lod++; voxelScale *= 2;
-                lodMax = f.lod_dist[lod];
+            Dda ray = gs.ray;
+            if (ray.dl >= f.lod_dist[lod]) {
+                dda_next_lod(ray, 1 << lod);
+                lod++;
             }
+            const float lodMax = f.lod_dist[lod];
             float myX = ray.tmx, myZ = ray.tmz, xEnd, zEnd;
             {
                 float x = ray.tmx, z = ray.tmz;
@@ -462,7 +491,7 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
             float myDl = __shfl_up_sync(gmask, myDn, 1, G);      // the previous cell's crossing is my last intersection
             if (gl == 0) myDl = ray.dl;
             const int cellX = ray.px + aK * ray.sx, cellZ = ray.pz + bK * ray.sz;
-            const bool oob = ((cellX & maskX) != cellX) || ((cellZ & maskZ) != cellZ);   // World.cs:135-138
+            const bool oob = ((cellX & (world.dim_x - 1)) != cellX) || ((cellZ & (world.dim_z - 1)) != cellZ);   // World.cs:135-138
             // first event in walk order: LOD switch before cell k (k >= 1), world exit at cell k, far clip after cell k (:613-615)
             const uint32_t swMask = GBALLOT(gl >= 1 && myDl >= lodMax), oobMask = GBALLOT(oob), farMask = GBALLOT(myDn >= farClip);
             const int kS = swMask ? __ffs(swMask) - 1 : G, kO = oobMask ? __ffs(oobMask) - 1 : G, kF = farMask ? __ffs(farMask) - 1 : G;
@@ -479,6 +508,8 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                 ray.px += aN * ray.sx; ray.pz += bN * ray.sz;
                 ray.dl = GSHFL(myDn, n - 1);
                 ray.dn = minf_(ray.tmx, ray.tmz);
+                __syncwarp(gmask); // every lane has read the batch's state
+                gs.ray = ray;
             }
             uint4 hdr = make_uint4(0, 0, 0, 0);
             if (gl < n) hdr = __ldg(world.lods[myLod].headers + myIdx);
@@ -491,21 +522,19 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
             uint32_t roundCols = 0u;      // batch cells whose runs are cached in the lanes
             uint32_t roundInvalid = 0u;   // lanes holding an invalid element (Length == 0), which ends its column (:445-447)
             int myBase = 0;               // batch lane c: first round lane of column c
-            // per-lane cached run: element fields, world-Y bounds, side span and cap span (none of it depends on the written-pixel state)
-            // (what only the commit of a span needs — colour indices, unrounded bounds, 1/w and u/w of both ends — is parked in
-            // shared memory, cache[field * G + lane], and read back by the whole group at the committing lane's index)
-            int r_ci = 0, r_sMin = 0, r_sMax = 0, r_cMin = 0, r_cMax = 0, r_capKind = 0;
-            bool r_sideClip = false, r_capClip = false;
+            // per-lane cached run: element, world-Y bounds, side span and cap span (none of it depends on the written-pixel state)
+            // (what only the commit of a span needs is parked in shared memory, cache[field * G + lane], and read back by the whole
+            // group at the committing lane's index: the cap colour (field 6) and, general kernel, the unrounded bounds, 1/w and u/w
+            // of both ends of the side span (fields 0-5); boundary-table kernel, the boundary's point on the last line (fields 0-2))
+            uint32_t r_el = 0u, r_side = 0u, r_cap = 0u; // RLEElement word; spans as span_pack
+            int r_capKind = 0;
             float r_eMin = 0.0f, r_eMax = 0.0f;
-            // FAST rounds: one BOUNDARY per lane (see world_transcode.h); the lane also owns the run between its boundary and the
-            // next lane's. Kept for the commit: the run's length, its cap colour and the boundary's point on the last line.
-            int r_len = 0; uint32_t r_capColor = 0u; float bFx = 0.0f, bFy = 0.0f, bFz = 0.0f;
             // Lanes of the round whose side / cap span held an unwritten pixel of the writable range when the round was formed. Written
             // pixels only grow and the writable range only shrinks, so these stay SUPERSETS of the spans that can still write: a
             // cached column none of whose lanes is set is inert (skipped like a culled one, see the hull comment below), and the
-            // commit loop looks at the set lanes only.
+            // commit loop looks at the set lanes only. A lane is set only if its run is solid and the span survived the near-plane
+            // clip, so nothing else of the round has to keep those two facts.
             uint32_t roundHotS = 0u, roundHotC = 0u;
-            bool r_solid = false;         // this lane holds a valid, non-air run
             const int myRunCount = (int)(hdr.y & 0xffffu);
 
             while (remaining) {
@@ -557,8 +586,9 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                     // lane L&3 of the group computes one of them (same operations as CameraData.cs:50-121), then they are shared.
                     const int L = gl & 3;
                     const float dLine = (L & 2) ? distNext : distLast; // :289-293 for this lane's line
-                    const F3 pMin = F3{planeBottom.x + planeDir.x * dLine, planeBottom.y + planeDir.y * dLine, planeBottom.z + planeDir.z * dLine};
-                    const F3 pMax = F3{planeTop.x + planeDir.x * dLine, planeTop.y + planeDir.y * dLine, planeTop.z + planeDir.z * dLine};
+                    const F3 pB = gs.planeBottom, pT = gs.planeTop, pD = gs.planeDir;
+                    const F3 pMin = F3{pB.x + pD.x * dLine, pB.y + pD.y * dLine, pB.z + pD.z * dLine};
+                    const F3 pMax = F3{pT.x + pD.x * dLine, pT.y + pD.y * dLine, pT.z + pD.z * dLine};
                     const bool A = pMin.x > pMin.z * rw.fb_max, B = pMax.x > pMax.z * rw.fb_max;
                     const bool C = pMin.x < pMin.z * rw.fb_min, D = pMax.x < pMax.z * rw.fb_min;
                     const bool clipped = (A && B) || (!A && !B && C && D);
@@ -606,8 +636,8 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                     const int writableMin = f2i(floorf(clippedMin));
                     const int writableMax = f2i(ceilf(clippedMax));
                     if (writableMax < rw.nf_min || writableMin > rw.nf_max) { terminated = true; cellsDone = c + 1; break; }
-                    if (writableMin > rw.nf_min) rw.nf_min = scan_up(rw.seen, writableMin, rw.orig_max);
-                    if (writableMax < rw.nf_max) rw.nf_max = scan_down(rw.seen, writableMax, rw.orig_min);
+                    if (writableMin > rw.nf_min) rw.nf_min = scan_up(rw.seen, writableMin, gs.orig_max);
+                    if (writableMax < rw.nf_max) rw.nf_max = scan_down(rw.seen, writableMax, gs.orig_min);
                     if (rw.nf_min > rw.nf_max) { terminated = true; cellsDone = c + 1; break; }
                 }
 
@@ -655,6 +685,7 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                         const uint32_t colOff = GSHFL(hdr.x, myCol);
                         const int colRuns = GSHFL(myRunCount, myCol);
                         const uint32_t* colElems = world.lods[cLod].elements + colOff; // one LOD per batch
+                        bool solidRun = false, sideClip = false, capClip = false; // valid non-air run; its side / cap span survived the clip
                         if (FAST) {
                             // ---- one boundary per lane: record k of the column (from the top, or from the bottom when iterating
                             // upwards) = {world-Y of the boundary, RLEElement below it}. The run of lane i lies between the boundaries
@@ -668,52 +699,52 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                             const uint32_t nextEl = __shfl_down_sync(gmask, rec.y, 1, G);
                             const bool laneRun = hasRun && k < colRuns && gl + 1 < totalRuns; // a boundary lane followed by the run's other boundary
                             const uint32_t el = laneRun ? (ITER > 0 ? rec.y : nextEl) : 0x0000ffffu; // others: air of length 0, never solid
-                            r_ci = (int)(short)(el & 0xffffu); r_len = (int)(short)(el >> 16);           // RLEElement World.cs:245-259
+                            r_el = el;
+                            const int ci = el_ci(el), len = el_len(el);
                             if (ITER > 0) { r_eMax = (float)yB; r_eMin = (float)nextY; } else { r_eMin = (float)yB; r_eMax = (float)nextY; }
 
                             STAMP(5);
-                            const F3 lMinLast = F3{planeBottom.x + planeDir.x * cDl, planeBottom.y + planeDir.y * cDl, planeBottom.z + planeDir.z * cDl}; // :289-293
-                            const F3 lMinNext = F3{planeBottom.x + planeDir.x * cDn, planeBottom.y + planeDir.y * cDn, planeBottom.z + planeDir.z * cDn};
-                            const F3 lMaxLast = F3{planeTop.x + planeDir.x * cDl, planeTop.y + planeDir.y * cDl, planeTop.z + planeDir.z * cDl};
-                            const F3 lMaxNext = F3{planeTop.x + planeDir.x * cDn, planeTop.y + planeDir.y * cDn, planeTop.z + planeDir.z * cDn};
+                            const F3 pB = gs.planeBottom, pT = gs.planeTop, pD = gs.planeDir;
+                            const F3 lMinLast = F3{pB.x + pD.x * cDl, pB.y + pD.y * cDl, pB.z + pD.z * cDl}; // :289-293
+                            const F3 lMinNext = F3{pB.x + pD.x * cDn, pB.y + pD.y * cDn, pB.z + pD.z * cDn};
+                            const F3 lMaxLast = F3{pT.x + pD.x * cDl, pT.y + pD.y * cDl, pT.z + pD.z * cDl};
+                            const F3 lMaxNext = F3{pT.x + pD.x * cDn, pT.y + pD.y * cDn, pT.z + pD.z * cDn};
                             const float portion = world.y_pow2 ? (float)yB * world.inv_dim_y : unlerpf(0.0f, worldMaxY, (float)yB); // :478-479
                             const F3 Fp = lerp3(lMinLast, lMaxLast, portion), Np = lerp3(lMinNext, lMaxNext, portion);
-                            bFx = Fp.x; bFy = Fp.y; bFz = Fp.z;
+                            cache[0 * G + gl] = __float_as_uint(Fp.x); cache[1 * G + gl] = __float_as_uint(Fp.y); cache[2 * G + gl] = __float_as_uint(Fp.z);
                             const bool fFront = !(Fp.y <= 0.0f), nFront = !(Np.y <= 0.0f); // in front of the near plane (CameraData.cs:126,143)
                             // which run's cap ends on this boundary: the run below it when it is seen from above (:549), the run above it
                             // when seen from below (:556); a run takes the first of the two that applies
                             const int bKind = portion < cameraPosYNormalized ? 1 : (portion > cameraPosYNormalized ? 2 : 0);
                             const float fpx = Fp.x / Fp.z;
                             const int fr = f2i(rintf(fpx));
-                            int bcMin = 0, bcMax = 0;
+                            uint32_t bcSpan = 0u;
                             if (bKind && fFront && nFront) { // :571-578
                                 const int nr = f2i(rintf(Np.x / Np.z));
-                                bcMin = nr; bcMax = fr;
-                                if (bcMin > bcMax) { bcMin = fr; bcMax = nr; }
+                                bcSpan = nr > fr ? span_pack(fr, nr) : span_pack(nr, fr);
                             }
                             const int flags = (fFront ? 1 : 0) | (nFront ? 2 : 0) | (bKind << 2);
                             const float nextFpx = __shfl_down_sync(gmask, fpx, 1, G);
                             const int nextFlags = __shfl_down_sync(gmask, flags, 1, G);
-                            const int nextCMin = __shfl_down_sync(gmask, bcMin, 1, G), nextCMax = __shfl_down_sync(gmask, bcMax, 1, G);
+                            const uint32_t nextCSpan = __shfl_down_sync(gmask, bcSpan, 1, G);
                             const bool nextFront = nextFlags & 1;
                             const int topKind = ITER > 0 ? bKind : (nextFlags >> 2), botKind = ITER > 0 ? (nextFlags >> 2) : bKind;
                             r_capKind = topKind == 1 ? 1 : (botKind == 2 ? 2 : 0); // :549,556
                             const bool capOwn = (r_capKind == 1) == (ITER > 0);      // the cap's boundary is this lane's (else the next lane's)
                             const bool capNFront = capOwn ? nFront : ((nextFlags & 2) != 0);
-                            r_sideClip = false; r_capClip = false;
-                            const bool solidRun = laneRun && r_ci >= 0;
-                            r_solid = solidRun;
+                            solidRun = laneRun && ci >= 0;
                             bool needExact = false;
+                            uint32_t capColor = 0u;
                             if (solidRun) {
                                 if (fFront && nextFront) {
                                     // both ends in front of the near plane: ClipHomogeneousCameraSpaceLine changes nothing
                                     const float fb = ITER > 0 ? nextFpx : fpx, ft = ITER > 0 ? fpx : nextFpx; // bottom / top end
                                     const int nextFr = f2i(rintf(nextFpx));
                                     const int rb = ITER > 0 ? nextFr : fr, rt = ITER > 0 ? fr : nextFr;
-                                    if (fb > ft) { r_sMin = rt; r_sMax = rb; } else { r_sMin = rb; r_sMax = rt; } // :496-502
-                                    r_sideClip = true;
+                                    r_side = fb > ft ? span_pack(rt, rb) : span_pack(rb, rt); // :496-502
+                                    sideClip = true;
                                     if (r_capKind) {
-                                        if (capNFront) { r_cMin = capOwn ? bcMin : nextCMin; r_cMax = capOwn ? bcMax : nextCMax; r_capClip = true; }
+                                        if (capNFront) { r_cap = capOwn ? bcSpan : nextCSpan; capClip = true; }
                                         else needExact = true;
                                     }
                                 } else if (!fFront && !nextFront) {
@@ -721,8 +752,9 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                                     // next-line end is in front (and then it is clipped)
                                     if (r_capKind && capNFront) needExact = true;
                                 } else needExact = true;
-                                if (r_capKind) r_capColor = __ldg(colElems + colRuns + 2 + (r_capKind == 1 ? r_ci : r_ci + r_len - 1)); // :553,560
+                                if (r_capKind) capColor = __ldg(colElems + colRuns + 2 + (r_capKind == 1 ? ci : ci + len - 1)); // :553,560
                             }
+                            cache[6 * G + gl] = capColor;
                             if (GBALLOT(needExact)) {
                                 EMU_STAT(8); // rounds with a run straddling the near plane
                                 // ---- a run straddles the near plane: the reference's per-run clipping (rare; columns next to the camera)
@@ -730,34 +762,36 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                                 const F3 nN = F3{__shfl_down_sync(gmask, Np.x, 1, G), __shfl_down_sync(gmask, Np.y, 1, G), __shfl_down_sync(gmask, Np.z, 1, G)};
                                 if (needExact) {
                                     F3 frontBottom = ITER > 0 ? nF : Fp, frontTop = ITER > 0 ? Fp : nF;
-                                    float uA = (float)r_len, uB = 0.0f;
-                                    r_sideClip = false; r_capClip = false;
+                                    float uA = (float)len, uB = 0.0f;
+                                    sideClip = false; capClip = false;
                                     if (clip_near_u(frontBottom, frontTop, uA, uB)) { // :489-502 (clips frontBottom/Top in place)
                                         float bfx = frontBottom.x / frontBottom.z, bfy = frontTop.x / frontTop.z;
                                         if (bfx > bfy) { float t = bfx; bfx = bfy; bfy = t; }
-                                        r_sMin = f2i(rintf(bfx)); r_sMax = f2i(rintf(bfy));
-                                        r_sideClip = true;
+                                        r_side = span_pack(f2i(rintf(bfx)), f2i(rintf(bfy)));
+                                        sideClip = true;
                                     }
                                     if (r_capKind) { // :554-578
                                         F3 secA = capOwn ? Np : nN, secB = r_capKind == 1 ? frontTop : frontBottom;
                                         if (clip_near(secA, secB)) {
-                                            r_cMin = f2i(rintf(secA.x / secA.z)); r_cMax = f2i(rintf(secB.x / secB.z));
-                                            if (r_cMin > r_cMax) { int t = r_cMin; r_cMin = r_cMax; r_cMax = t; }
-                                            r_capClip = true;
+                                            const int a = f2i(rintf(secA.x / secA.z)), b = f2i(rintf(secB.x / secB.z));
+                                            r_cap = a > b ? span_pack(b, a) : span_pack(a, b);
+                                            capClip = true;
                                         }
                                     }
                                 }
                             }
+                            __syncwarp(gmask);
                         } else {
                             uint32_t el = 0u;
                             if (hasRun) el = __ldg(colElems + (ITER > 0 ? 1 + k : colRuns - k));
-                            r_ci = (int)(short)(el & 0xffffu); r_len = (int)(short)(el >> 16); // RLEElement World.cs:245-259
-                            roundInvalid = GBALLOT(hasRun && r_len == 0);  // an invalid element (Length == 0) ends its column (:445-447)
+                            r_el = el;
+                            const int ci = el_ci(el), len = el_len(el);
+                            roundInvalid = GBALLOT(hasRun && len == 0);  // an invalid element (Length == 0) ends its column (:445-447)
                             // lanes of my column from its start up to me, and whether an invalid element precedes me there
                             const uint32_t mineUpToMe = ((2u << gl) - 1u) & ~((1u << myStart) - 1u);
                             const bool valid = hasRun && !(roundInvalid & mineUpToMe);
-                            r_solid = valid && r_ci >= 0;
-                            const int span = valid ? r_len * cScale : 0;
+                            solidRun = valid && ci >= 0;
+                            const int span = valid ? len * cScale : 0;
                             int sum = span;
     #pragma unroll
                             for (int o = 1; o < G; o <<= 1) { int t = __shfl_up_sync(gmask, sum, o, G); if (gl >= o) sum += t; }
@@ -768,11 +802,12 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                             else          { r_eMin = (float)(inclCol - span); r_eMax = (float)inclCol; }
 
                             STAMP(5);
-                            const F3 lMinLast = F3{planeBottom.x + planeDir.x * cDl, planeBottom.y + planeDir.y * cDl, planeBottom.z + planeDir.z * cDl}; // :289-293
-                            const F3 lMinNext = F3{planeBottom.x + planeDir.x * cDn, planeBottom.y + planeDir.y * cDn, planeBottom.z + planeDir.z * cDn};
-                            const F3 lMaxLast = F3{planeTop.x + planeDir.x * cDl, planeTop.y + planeDir.y * cDl, planeTop.z + planeDir.z * cDl};
-                            const F3 lMaxNext = F3{planeTop.x + planeDir.x * cDn, planeTop.y + planeDir.y * cDn, planeTop.z + planeDir.z * cDn};
-                            r_sideClip = false; r_capClip = false; r_capKind = 0;
+                            const F3 pB = gs.planeBottom, pT = gs.planeTop, pD = gs.planeDir;
+                            const F3 lMinLast = F3{pB.x + pD.x * cDl, pB.y + pD.y * cDl, pB.z + pD.z * cDl}; // :289-293
+                            const F3 lMinNext = F3{pB.x + pD.x * cDn, pB.y + pD.y * cDn, pB.z + pD.z * cDn};
+                            const F3 lMaxLast = F3{pT.x + pD.x * cDl, pT.y + pD.y * cDl, pT.z + pD.z * cDl};
+                            const F3 lMaxNext = F3{pT.x + pD.x * cDn, pT.y + pD.y * cDn, pT.z + pD.z * cDn};
+                            r_capKind = 0;
                             {
                                 float bfx = 0.0f, bfy = 0.0f, uvAx = 0.0f, uvAy = 0.0f, uvBx = 0.0f, uvBy = 0.0f;
                                 int capIdx = 0;
@@ -782,11 +817,11 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                                 F3 frontTop = lerp3(lMinLast, lMaxLast, portionTop);
                                 // which cap, if any, depends on the camera height only (:549,556); its flat colour (:553,560) is fetched
                                 // now, while the divisions below run, and parked in the cache
-                                if (portionTop < cameraPosYNormalized) { r_capKind = 1; capIdx = r_ci; }
-                                else if (portionBottom > cameraPosYNormalized) { r_capKind = 2; capIdx = r_ci + r_len - 1; }
+                                if (portionTop < cameraPosYNormalized) { r_capKind = 1; capIdx = ci; }
+                                else if (portionBottom > cameraPosYNormalized) { r_capKind = 2; capIdx = ci + len - 1; }
                                 uint32_t capColor = 0u;
-                                if (r_capKind && valid && r_ci >= 0) capColor = __ldg(colElems + colRuns + 2 + capIdx);
-                                float uA = (float)r_len, uB = 0.0f;
+                                if (r_capKind && solidRun) capColor = __ldg(colElems + colRuns + 2 + capIdx);
+                                float uA = (float)len, uB = 0.0f;
                                 if (clip_near_u(frontBottom, frontTop, uA, uB)) { // :489-502 (clips frontBottom/Top in place)
                                     uvAx = 1.0f / frontBottom.z; uvAy = uA / frontBottom.z;
                                     uvBx = 1.0f / frontTop.z;    uvBy = uB / frontTop.z;
@@ -796,28 +831,28 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                                         t = uvAx; uvAx = uvBx; uvBx = t;
                                         t = uvAy; uvAy = uvBy; uvBy = t;
                                     }
-                                    r_sMin = f2i(rintf(bfx)); r_sMax = f2i(rintf(bfy));
-                                    r_sideClip = true;
+                                    r_side = span_pack(f2i(rintf(bfx)), f2i(rintf(bfy)));
+                                    sideClip = true;
                                 }
                                 if (r_capKind) { // :554-578
                                     const float portion = r_capKind == 1 ? portionTop : portionBottom;
                                     F3 secA = lerp3(lMinNext, lMaxNext, portion), secB = r_capKind == 1 ? frontTop : frontBottom;
                                     if (clip_near(secA, secB)) {
-                                        r_cMin = f2i(rintf(secA.x / secA.z)); r_cMax = f2i(rintf(secB.x / secB.z));
-                                        if (r_cMin > r_cMax) { int t = r_cMin; r_cMin = r_cMax; r_cMax = t; }
-                                        r_capClip = true;
+                                        const int a = f2i(rintf(secA.x / secA.z)), b = f2i(rintf(secB.x / secB.z));
+                                        r_cap = a > b ? span_pack(b, a) : span_pack(a, b);
+                                        capClip = true;
                                     }
                                 }
                                 cache[0 * G + gl] = __float_as_uint(bfx);  cache[1 * G + gl] = __float_as_uint(bfy);
                                 cache[2 * G + gl] = __float_as_uint(uvAx); cache[3 * G + gl] = __float_as_uint(uvAy);
                                 cache[4 * G + gl] = __float_as_uint(uvBx); cache[5 * G + gl] = __float_as_uint(uvBy);
-                                cache[6 * G + gl] = (uint32_t)r_len;       cache[7 * G + gl] = capColor;
+                                cache[6 * G + gl] = capColor;
                                 __syncwarp(gmask);
                             }
                         }
                         STAMP(6);
-                        roundHotS = GBALLOT(r_solid && r_sideClip && span_would_write(rw, r_sMin, r_sMax));
-                        roundHotC = GBALLOT(r_solid && r_capClip && span_would_write(rw, r_cMin, r_cMax));
+                        roundHotS = GBALLOT(solidRun && sideClip && span_would_write(rw, span_lo(r_side), span_hi(r_side)));
+                        roundHotC = GBALLOT(solidRun && capClip && span_would_write(rw, span_lo(r_cap), span_hi(r_cap)));
                         STAMP(4);
                     }
 
@@ -827,29 +862,29 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                     const bool inCol = (colMask >> gl) & 1u;
                     const uint32_t invalidHere = roundInvalid & colMask;
                     const int endValid = invalidHere ? __ffs(invalidHere) - 1 : base + runsHere; // first lane past the valid runs
-                    const bool solid = inCol && gl < endValid && r_ci >= 0; // valid and !IsAir
+                    const bool solid = inCol && gl < endValid && el_ci(r_el) >= 0; // valid and !IsAir
                     const bool above = r_eMin > worldBoundsMax, below = r_eMax < worldBoundsMin;
                     const bool isBreak = solid && (ITER > 0 ? (!above && below) : above); // :461-475 (above is tested first)
                     const uint32_t breakMask = GBALLOT(isBreak);
                     const int endVisit = breakMask ? __ffs(breakMask) : endValid;           // the breaking run itself was dereferenced
                     if (invalidHere | breakMask) colStop = true;
                     const bool active = solid && gl < endVisit && !above && !below;
-                    const bool sideOk = active && r_sideClip;
-                    const bool capOk = active && r_capClip &&
-                                       (r_capKind == 1 ? !(r_eMax > worldBoundsMax) : !(r_eMin < worldBoundsMin)); // :549-565
+                    // (the clip of the side / cap span is part of roundHotS / roundHotC)
+                    const bool capOk = active && (r_capKind == 1 ? !(r_eMax > worldBoundsMax) : !(r_eMin < worldBoundsMin)); // :549-565
 
                     STAMP(6);
                     // ---- commit, in reference order (side of run j, cap of run j, side of run j+1, ...), only the spans that still
                     // hold an unwritten pixel; everything ordered before the committed span is a no-op now and stays one (written
                     // pixels only grow, the writable range only shrinks), so it is retired with it.
-                    uint32_t candS = GBALLOT(sideOk) & roundHotS, candC = GBALLOT(capOk) & roundHotC;
+                    uint32_t candS = GBALLOT(active) & roundHotS, candC = GBALLOT(capOk) & roundHotC;
                     int visitedHere = endVisit - base;
                     while (candS | candC) {
                         const int jS = candS ? __ffs(candS) - 1 : 64, jC = candC ? __ffs(candC) - 1 : 64;
                         const bool isCap = jC < jS;
                         const int j = isCap ? jC : jS;
                         if (isCap) candC &= candC - 1u; else candS &= candS - 1u;
-                        int bMin = GSHFL(isCap ? r_cMin : r_sMin, j), bMax = GSHFL(isCap ? r_cMax : r_sMax, j);
+                        const uint32_t span = GSHFL(isCap ? r_cap : r_side, j);
+                        int bMin = span_lo(span), bMax = span_hi(span);
                         EMU_STAT(5); // commit candidates examined
                         STAMP(8);
                         if (!span_would_write(rw, bMin, bMax)) { STAMP(6); continue; } // written over / cut off since the round was formed
@@ -858,23 +893,24 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                         STAMP(9);
                         reduce_pixel_horizon(rw, bMin, bMax); // :507-517 / :583-593
                         STAMP(10);
+                        uint32_t* const row = gs.row;
                         if (isCap) {
-                            const uint32_t color = FAST ? GSHFL(r_capColor, j) : cache[7 * G + j];
+                            const uint32_t color = cache[6 * G + j];
                             for (int y = bMin + gl; y <= bMax; y += G) // :595-602
                                 if (!((rw.seen[y >> 5] >> (y & 31)) & 1u)) row[y] = color;
                         } else {
                             STAMP(11);
                             float jbfx, jbfy, jAx, jAy, jBx, jBy;
-                            int jLen;
-                            const int jCi = GSHFL(r_ci, j);
+                            const uint32_t jEl = GSHFL(r_el, j);
+                            const int jCi = el_ci(jEl), jLen = el_len(jEl);
                             if (FAST) {
                                 // the perspective-correct u of :490-491,525-530 is needed only now, for the one span that writes, and
                                 // only if the run is longer than one voxel (clamp(floor(u), 0, Length - 1) is 0 otherwise): rebuild the
                                 // span's ends from the boundary points of lanes j and j + 1 exactly as :478-502 does
-                                jLen = GSHFL(r_len, j);
                                 jbfx = jbfy = jAx = jAy = jBx = jBy = 0.0f;
                                 if (jLen > 1) {
-                                    const F3 pj = F3{GSHFL(bFx, j), GSHFL(bFy, j), GSHFL(bFz, j)}, pn = F3{GSHFL(bFx, j + 1), GSHFL(bFy, j + 1), GSHFL(bFz, j + 1)};
+                                    const F3 pj = F3{__uint_as_float(cache[0 * G + j]), __uint_as_float(cache[1 * G + j]), __uint_as_float(cache[2 * G + j])};
+                                    const F3 pn = F3{__uint_as_float(cache[0 * G + j + 1]), __uint_as_float(cache[1 * G + j + 1]), __uint_as_float(cache[2 * G + j + 1])};
                                     F3 frontBottom = ITER > 0 ? pn : pj, frontTop = ITER > 0 ? pj : pn;
                                     float uA = (float)jLen, uB = 0.0f;
                                     clip_near_u(frontBottom, frontTop, uA, uB);
@@ -891,7 +927,6 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
                                 jbfx = __uint_as_float(cache[0 * G + j]); jbfy = __uint_as_float(cache[1 * G + j]);
                                 jAx = __uint_as_float(cache[2 * G + j]); jAy = __uint_as_float(cache[3 * G + j]);
                                 jBx = __uint_as_float(cache[4 * G + j]); jBy = __uint_as_float(cache[5 * G + j]);
-                                jLen = (int)cache[6 * G + j];
                             }
                             STAMP(12);
                             for (int y = bMin + gl; y <= bMax; y += G) { // :519-533
@@ -927,13 +962,15 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
         STAMP(7);
         // WriteSkybox :699-708 — :248,268,323,401,419,537,606,619 all end here
         __syncwarp(gmask);
-        for (int y = rw.orig_min + gl; y <= rw.orig_max; y += G)
+        uint32_t* const row = gs.row;
+        const int origMin = gs.orig_min, origMax = gs.orig_max;
+        for (int y = origMin + gl; y <= origMax; y += G)
             if (!((rw.seen[y >> 5] >> (y & 31)) & 1u)) row[y] = SKYBOX_ARGB;
         if (COUNTERS) {
-            for (int w = (rw.orig_min >> 5) + gl; w <= (rw.orig_max >> 5); w += G) {
+            for (int w = (origMin >> 5) + gl; w <= (origMax >> 5); w += G) {
                 uint32_t m = FULL_MASK;
-                if (w == (rw.orig_min >> 5)) m &= mask_from(rw.orig_min);
-                if (w == (rw.orig_max >> 5)) m &= mask_to(rw.orig_max);
+                if (w == (origMin >> 5)) m &= mask_from(origMin);
+                if (w == (origMax >> 5)) m &= mask_to(origMax);
                 acc.px_sky += __popc(~rw.seen[w] & m);
             }
         }
@@ -954,6 +991,8 @@ phase1_kernel(const __grid_constant__ cvxd_world world, const __grid_constant__ 
 #undef GBALLOT
 #undef GSHFL
 #undef worldMaxY
+#undef farClip
+#undef camY
 #undef cameraPosYNormalized
 }
 
@@ -1305,8 +1344,7 @@ template <int G>
 static cudaError_t launch_phase1_g(const cvxd_world& world, const cvxd_frame& frame, int n, cudaStream_t stream) {
     constexpr int groupsPerCta = CVXD_THREADS_PER_CTA / G;
     const int blocks = (n + groupsPerCta - 1) / groupsPerCta;
-    const int seenWords = ((frame.width > frame.height ? frame.width : frame.height) + 31) >> 5;
-    const size_t smem = (size_t)groupsPerCta * (seenWords + 9 * G) * sizeof(uint32_t);
+    const size_t smem = phase1_smem_bytes(G, frame.width, frame.height);
     // FAST: the boundary-table kernel, for regular worlds (world_transcode.h)
     const bool fast = world.regular && !frame.general_path;
 #define CVXD_P1(C, T, F) do { \

@@ -108,8 +108,7 @@ int emu_phase1(const emu_world* w, const cvx_frame_setup* setup, int W, int H, u
     if (group != 8 && group != 16 && group != 32) group = 32;
     const int groupsPerCta = CVXD_THREADS_PER_CTA / group;
     const int blocks = (n + groupsPerCta - 1) / groupsPerCta;
-    const int seenWords = ((W > H ? W : H) + 31) >> 5;
-    const size_t smemWords = (size_t)groupsPerCta * (seenWords + 9 * group) + 64;
+    const size_t smemWords = phase1_smem_bytes(group, W, H) / sizeof(uint32_t) + 64;
     LaunchArgs args{&w->w, &f, variant, group, counters != nullptr};
     std::atomic<int> next{0};
     if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
