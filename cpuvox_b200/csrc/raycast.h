@@ -107,7 +107,8 @@ __device__ __forceinline__ void cvxr_cast(const cvxd_world& w, int lod, const cv
     }
     out.hit = 0;
     const int n[3] = {w.dim_x >> lod, w.dim_y >> lod, w.dim_z >> lod};
-    const float dimf[3] = {(float)w.dim_x, (float)w.dim_y, (float)w.dim_z};
+    // the box of the LOD's cells: n << lod is the world size along x and z, and short of dim_y by dim_y mod 2^lod
+    const float dimf[3] = {(float)(n[0] << lod), (float)(n[1] << lod), (float)(n[2] << lod)};
     // box entry: slab test, axes in the order x, z, y (ties of the entry distance go to the earlier axis)
     float tEnter = -inf, tExit = inf;
     int entry = -1;

@@ -88,13 +88,13 @@ void cast(const World& w, int lod, const Ray& r, Hit& out) {
     const float* o = r.origin;
     const float maxd = r.max_distance;
     const int n[3] = {w.dims[0] >> lod, w.dims[1] >> lod, w.dims[2] >> lod};
-    // 2. enter the box [0,dim]^3
+    // 2. enter the box of the LOD's cells, [0, n_i << lod] per axis (short of dim_y when 2^lod does not divide it)
     float tEnter = -INFINITY, tExit = INFINITY;
     int entry = -1;
     const int order[3] = {0, 2, 1};
     for (int q = 0; q < 3; q++) {
         const int i = order[q];
-        const float dim = (float)w.dims[i];
+        const float dim = (float)(n[i] << lod);
         if (step[i] == 0) {
             if (!(o[i] >= 0.0f && o[i] < dim)) return;
             continue;
