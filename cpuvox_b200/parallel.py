@@ -5,8 +5,7 @@ raybuffer row (DrawSegmentRayJob.cs:106,199), so
   * batched views (BASELINE config 5) are dealt round-robin to ranks, no per-frame exchange at all;
   * a single large view (configs 3, 4) is cut into contiguous flat-ray ranges in RaySetupJob order (DrawSegmentRayJob.cs:12-40);
     each rank runs Phase 1 for its rays and Phase 2 only for the screen pixels those rays feed, storing them straight into
-    the root's framebuffer through a CUDA-IPC mapping (NVLink peer stores; the gather is the kernel's own stores). A
-    `reduce` fallback sums zero-initialised, disjoint framebuffers with NCCL instead.
+    the root's framebuffer through a CUDA-IPC mapping (NVLink peer stores; the gather is the kernel's own stores).
 torch is used for process-group plumbing only; all rendering goes through the C ABI.
 """
 from __future__ import annotations
@@ -96,18 +95,15 @@ class ShardedRenderManager:
 
     gather: "p2p"    one view at a time: peer stores into the root's framebuffer, a host barrier per view;
             "ring"   a stream of views: peer stores into a ring of framebuffers on the root, all ordering between ranks on the
-                     device (flag words polled by tiny kernels), no host barrier and no collective between views;
-            "reduce" fallback: zero-initialised disjoint framebuffers summed with ncclReduce."""
+                     device (flag words polled by tiny kernels), no host barrier and no collective between views."""
 
     def __init__(self, device: int, rank: int, world_size: int, gather: str = "p2p", group=None, ring_slots: int = 4):
-        if gather not in ("p2p", "reduce", "ring"):
-            raise ValueError("gather must be 'p2p', 'ring' or 'reduce'")
+        if gather not in ("p2p", "ring"):
+            raise ValueError("gather must be 'p2p' or 'ring'")
         self.rm = RenderManager(device)
         self.device, self.rank, self.world_size, self.gather, self.group = device, rank, world_size, gather, group
         self.ring_slots = ring_slots
         self._root_frame_ptr = 0      # mapped pointer to rank 0's framebuffer (p2p, rank != 0)
-        self._frame_tensor = None     # torch int32 tensor aliasing this rank's framebuffer (reduce)
-        self._stream = None
         self._next_view = 0           # ring: running view index, the same on every rank
         self._ring_ready = False
 
@@ -115,11 +111,10 @@ class ShardedRenderManager:
         self.rm.upload_world(world)
 
     def set_resolution(self, width: int, height: int):
-        import torch
         import torch.distributed as dist
 
         same = width == self.rm.width and height == self.rm.height
-        if same and (self._root_frame_ptr or self._frame_tensor is not None or self._ring_ready or self.world_size == 1):
+        if same and (self._root_frame_ptr or self._ring_ready or self.world_size == 1):
             return
         if self.world_size > 1 and not same:
             # peers close their mappings of the root's memory BEFORE the root reallocates it (CUDA IPC rule), then everyone moves on
@@ -142,21 +137,13 @@ class ShardedRenderManager:
             dist.broadcast_object_list(handle, src=0, group=self.group)
             if self.rank != 0:
                 self._root_frame_ptr = self.rm.ipc_open(handle[0])
-        elif self.gather == "ring":
+        else:
             handle = [self.rm.ring_create(self.ring_slots, self.world_size) if self.rank == 0 else None]
             dist.broadcast_object_list(handle, src=0, group=self.group)
             if self.rank != 0:
                 self.rm.ring_open(handle[0], self.ring_slots, self.world_size)
             self._ring_ready = True
             self._next_view = 0
-        else:
-            # render into a torch-owned buffer on torch's stream so NCCL sees the same memory and ordering
-            self._frame_tensor = torch.zeros(width * height, dtype=torch.int32, device=f"cuda:{self.device}")
-            if self._stream is None:  # an explicit stream: torch's default stream is the NULL handle (= "own stream" for cvx_set_stream)
-                self._stream = torch.cuda.Stream(self.device)
-            torch.cuda.set_stream(self._stream)
-            self.rm.set_stream(self._stream.cuda_stream)
-            self.rm.set_external_frame(self._frame_tensor.data_ptr())
 
     def draw_world_sharded(self, pose: CameraPose, weights: Optional[Sequence[float]] = None) -> FrameSetup:
         """Single view, rays sharded: after the call (and its barrier) rank 0's framebuffer holds the whole frame."""
@@ -174,19 +161,13 @@ class ShardedRenderManager:
         if self.gather == "ring":
             self.draw_views_sharded([pose], weights=[weights])
             return setup
-        if self.gather == "p2p":
-            # the previous view is final on the root only after the barrier that ended it; whoever reads or presents it there must do
-            # so before entering this call — this barrier keeps a fast rank from storing into it any earlier than that
-            dist.barrier(group=self.group)
-            rm.draw_rays(setup, begin, end)
-            rm.blit_owned(setup, begin, end, self._root_frame_ptr)
-            rm.sync()
-            dist.barrier(group=self.group)  # every rank's peer stores have landed
-        else:
-            self._frame_tensor.zero_()
-            rm.draw_rays(setup, begin, end)
-            rm.blit_owned(setup, begin, end, 0)
-            dist.reduce(self._frame_tensor, dst=0, op=dist.ReduceOp.SUM, group=self.group)  # disjoint pixels: sum == copy
+        # the previous view is final on the root only after the barrier that ended it; whoever reads or presents it there must do
+        # so before entering this call — this barrier keeps a fast rank from storing into it any earlier than that
+        dist.barrier(group=self.group)
+        rm.draw_rays(setup, begin, end)
+        rm.blit_owned(setup, begin, end, self._root_frame_ptr)
+        rm.sync()
+        dist.barrier(group=self.group)  # every rank's peer stores have landed
         return setup
 
     def draw_views_sharded(self, poses: Sequence[CameraPose], dst: Optional[np.ndarray] = None, weights: Optional[Sequence] = None,
@@ -245,11 +226,7 @@ class ShardedRenderManager:
         return mine
 
     def read_frame(self) -> np.ndarray:
-        """The last single view on the root (p2p / reduce). Ring views are delivered through draw_views_sharded(dst=...)."""
-        if self._frame_tensor is not None:
-            import torch
-            torch.cuda.current_stream(self.device).synchronize()
-            return self._frame_tensor.cpu().numpy().view(np.uint32).reshape(self.rm.height, self.rm.width)
+        """The last single view on the root (p2p). Ring views are delivered through draw_views_sharded(dst=...)."""
         return self.rm.read_frame()
 
     def destroy(self):
