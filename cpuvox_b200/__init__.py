@@ -6,6 +6,7 @@ shared library has not been built — there is no CPU or Python fallback.
 """
 from .native import LIB_PATH, CvxError, FrameSetup, LOD_LEVELS  # noqa: F401
 from .host import (  # noqa: F401
+    BOX_DTYPE,
     RAY_DTYPE,
     RAY_HIT_DTYPE,
     SKYBOX_ARGB,
@@ -18,6 +19,7 @@ from .host import (  # noqa: F401
     benchmark_path,
     benchmark_pose,
     frame_setup,
+    make_boxes,
     make_rays,
     screen_ray,
     setup_lods,

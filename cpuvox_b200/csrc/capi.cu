@@ -27,6 +27,7 @@ static_assert(sizeof(cvx_counters) == sizeof(cvxd_counters), "counter layout");
 static_assert(CVX_LOD_LEVELS == CVXD_LODS, "lod levels");
 static_assert(sizeof(cvx_ray) == sizeof(cvxd_ray) && sizeof(cvx_ray) == 32, "ray layout");
 static_assert(sizeof(cvx_ray_hit) == sizeof(cvxd_ray_hit) && sizeof(cvx_ray_hit) == 32, "ray hit layout");
+static_assert(sizeof(cvx_box) == sizeof(cvxd_box) && sizeof(cvx_box) == 48, "box layout");
 
 #define CVX_MAX_SLOTS 16
 #define CVX_DEFAULT_SLOTS 6
@@ -95,7 +96,7 @@ struct cvx_ctx {
     size_t ringFrameBytes = 0;
     int groupSize = 0;                  // lanes per ray in phase 1: 0 = auto, 8, 16, 32
     int generalPath = 0;                // 1 = never use the boundary-table kernel
-    void* rayScratch = nullptr;         // cvx_raycast with host arrays: rays then hits, grown to the largest call
+    void* rayScratch = nullptr;         // cvx_raycast / cvx_sweep with host arrays: queries then hits, grown to the largest call
     size_t rayScratchBytes = 0;
     std::string error;
 };
@@ -840,24 +841,28 @@ int cvx_world_build_from_mesh(cvx_ctx* ctx, const float* positions, const uint8_
     return CVX_OK;
 }
 
-// Ray queries (raycast.h, raycast_kernels.cu): the kernel reads the world tables the context holds at the time of the call, on the
-// context's stream, so it follows any draw or batch join queued there and a later world replacement (which synchronises that stream
-// before freeing the old tables) cannot pull them from under it.
-int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device) {
+// Ray and box queries (raycast.h, raycast_kernels.cu): the kernel reads the world tables the context holds at the time of the call, on
+// the context's stream, so it follows any draw or batch join queued there and a later world replacement (which synchronises that
+// stream before freeing the old tables) cannot pull them from under it. Host arrays go through one scratch shared by both queries.
+namespace {
+using query_launch = cudaError_t (*)(const cvxd_world&, int, const void*, cvxd_ray_hit*, int, bool, cudaStream_t);
+
+int world_query(cvx_ctx* ctx, const char* what, const void* queries, size_t query_bytes, int32_t n, int32_t lod, cvx_ray_hit* out,
+                int32_t on_device, query_launch launch) {
     if (!ctx) return CVX_ERR_INVALID_ARGUMENT;
     if (ctx->world.lod_count <= 0) return fail(ctx, CVX_ERR_NO_WORLD, "no world uploaded");
     if (lod < 0 || lod >= CVX_LOD_LEVELS || !ctx->world.lods[lod].headers) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "LOD %d is not uploaded", lod);
     if (n < 0) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "n = %d < 0", n);
-    if (n > 0 && (!rays || !out)) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "rays or hits is NULL");
+    if (n > 0 && (!queries || !out)) return fail(ctx, CVX_ERR_INVALID_ARGUMENT, "%s or hits is NULL", what);
     if (n == 0) return CVX_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     const bool bounds = ctx->lod[lod].regular && !ctx->generalPath;
     if (on_device) {
-        CU(ctx, cvxd_launch_raycast(ctx->world, lod, (const cvxd_ray*)rays, (cvxd_ray_hit*)out, n, bounds, ctx->stream));
+        CU(ctx, launch(ctx->world, lod, queries, (cvxd_ray_hit*)out, n, bounds, ctx->stream));
         ctx->launches++;
         return CVX_OK;
     }
-    const size_t rayBytes = (size_t)n * sizeof(cvx_ray), need = rayBytes + (size_t)n * sizeof(cvx_ray_hit);
+    const size_t inBytes = (size_t)n * query_bytes, need = inBytes + (size_t)n * sizeof(cvx_ray_hit);
     if (need > ctx->rayScratchBytes) {
         CU(ctx, cudaStreamSynchronize(ctx->stream));
         free_ray_scratch(ctx);
@@ -865,14 +870,29 @@ int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_r
         if (e != cudaSuccess) { ctx->rayScratch = nullptr; return fail(ctx, cvx_code(e), "ray scratch allocation failed: %s", cudaGetErrorString(e)); }
         ctx->rayScratchBytes = need;
     }
-    cvxd_ray* dRays = (cvxd_ray*)ctx->rayScratch;
-    cvxd_ray_hit* dHits = (cvxd_ray_hit*)((uint8_t*)ctx->rayScratch + rayBytes);
-    CU(ctx, cudaMemcpyAsync(dRays, rays, rayBytes, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cvxd_launch_raycast(ctx->world, lod, dRays, dHits, n, bounds, ctx->stream));
+    void* dIn = ctx->rayScratch;
+    cvxd_ray_hit* dHits = (cvxd_ray_hit*)((uint8_t*)ctx->rayScratch + inBytes);
+    CU(ctx, cudaMemcpyAsync(dIn, queries, inBytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, launch(ctx->world, lod, dIn, dHits, n, bounds, ctx->stream));
     ctx->launches++;
     CU(ctx, cudaMemcpyAsync(out, dHits, (size_t)n * sizeof(cvx_ray_hit), cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return CVX_OK;
+}
+} // namespace
+
+int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device) {
+    return world_query(ctx, "rays", rays, sizeof(cvx_ray), n, lod, out, on_device,
+                       [](const cvxd_world& w, int l, const void* q, cvxd_ray_hit* h, int m, bool b, cudaStream_t s) {
+                           return cvxd_launch_raycast(w, l, (const cvxd_ray*)q, h, m, b, s);
+                       });
+}
+
+int cvx_sweep(cvx_ctx* ctx, const cvx_box* boxes, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device) {
+    return world_query(ctx, "boxes", boxes, sizeof(cvx_box), n, lod, out, on_device,
+                       [](const cvxd_world& w, int l, const void* q, cvxd_ray_hit* h, int m, bool b, cudaStream_t s) {
+                           return cvxd_launch_sweep(w, l, (const cvxd_box*)q, h, m, b, s);
+                       });
 }
 
 int cvx_read_frame(cvx_ctx* ctx, void* dst_argb, int64_t bytes) {

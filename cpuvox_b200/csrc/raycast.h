@@ -82,6 +82,25 @@ __device__ __forceinline__ int cvxr_first_solid_bounds(const cvxd_lod& L, uint4 
     return -1;
 }
 
+// Step 1 of DESIGN.md §3.5 (shared by §3.6): normalise `dir` into d, with inv_i = 1/d_i and step_i = sign(d_i) per axis; an axis
+// whose component is 0 or too small to invert does not move (d_i = inv_i = 0, step_i = 0). False when the squared length is 0 or
+// not finite (the query is invalid).
+__device__ __forceinline__ bool cvxr_normalise(const float dir[3], float d[3], float inv[3], int step[3]) {
+    const float len2 = dir[0] * dir[0] + dir[1] * dir[1] + dir[2] * dir[2];
+    if (!(len2 > 0.0f) || !cvxr_finite(len2)) return false;
+    const float invLen = 1.0f / sqrtf(len2);
+    for (int i = 0; i < 3; i++) {
+        d[i] = dir[i] * invLen;
+        inv[i] = 0.0f; step[i] = 0;
+        if (d[i] != 0.0f) {
+            const float v = 1.0f / d[i];
+            if (cvxr_finite(v)) { inv[i] = v; step[i] = d[i] > 0.0f ? 1 : -1; }
+            else d[i] = 0.0f;
+        }
+    }
+    return true;
+}
+
 // One ray at LOD `lod` (uploaded). use_bounds: read runs from the boundary records (the LOD is regular) instead of the element area.
 __device__ __forceinline__ void cvxr_cast(const cvxd_world& w, int lod, const cvxd_ray& r, bool use_bounds, cvxd_ray_hit& out) {
     out.hit = -1; out.face = 0; out.cell[0] = out.cell[1] = out.cell[2] = 0; out.distance = 0.0f; out.color = 0; out.steps = 0;
@@ -91,20 +110,9 @@ __device__ __forceinline__ void cvxr_cast(const cvxd_world& w, int lod, const cv
     if (!cvxr_finite(o[0]) || !cvxr_finite(o[1]) || !cvxr_finite(o[2]) || !cvxr_finite(r.direction[0]) || !cvxr_finite(r.direction[1]) ||
         !cvxr_finite(r.direction[2]) || !(maxd == inf || cvxr_finite(maxd)))
         return;
-    const float len2 = r.direction[0] * r.direction[0] + r.direction[1] * r.direction[1] + r.direction[2] * r.direction[2];
-    if (!(len2 > 0.0f) || !cvxr_finite(len2)) return;
-    const float invLen = 1.0f / sqrtf(len2);
     float d[3], inv[3];
     int step[3];
-    for (int i = 0; i < 3; i++) {
-        d[i] = r.direction[i] * invLen;
-        inv[i] = 0.0f; step[i] = 0;
-        if (d[i] != 0.0f) {
-            const float v = 1.0f / d[i];
-            if (cvxr_finite(v)) { inv[i] = v; step[i] = d[i] > 0.0f ? 1 : -1; }
-            else d[i] = 0.0f;             // a component too small to invert: the ray does not move along this axis
-        }
-    }
+    if (!cvxr_normalise(r.direction, d, inv, step)) return;
     out.hit = 0;
     const int n[3] = {w.dim_x >> lod, w.dim_y >> lod, w.dim_z >> lod};
     // the box of the LOD's cells: n << lod is the world size along x and z, and short of dim_y by dim_y mod 2^lod
@@ -198,7 +206,181 @@ __device__ __forceinline__ void cvxr_cast(const cvxd_world& w, int lod, const cv
     }
 }
 
+/*
+ * Swept boxes (cvx_sweep, DESIGN.md §3.6): how far an axis-aligned box moves along a direction before it touches a solid cell.
+ * Per axis, cell k's window is the open interval (enter, exit) of times at which the open box overlaps the cell's slab, with
+ * lo = (float)(k << j) - h and hi = (float)((k+1) << j) + h; a cell is a candidate when the three windows meet after 0 and enter by
+ * max_distance, and the solid candidate with the smallest key (t*, overlapping first, cx, cz, cy) is the result.
+ *
+ * Along the direction of travel of a moving axis both enter(k) and exit(k) are non-decreasing (every operation rounds
+ * monotonically), so every condition but "enter < exit of one cell" selects a prefix or a suffix of an axis's cells: the walk below
+ * visits the slabs of the XZ major axis in travel order, in each the interval of minor cells, and in each column the interval of
+ * y cells, each interval found from a position estimate fixed up against the exact expressions. The cost grows with the box's XZ
+ * footprint in cells (one header per column it sweeps) and with its length of travel; there is no size cap.
+ */
+struct cvxd_box { float center[3]; float max_distance; float direction[3]; int32_t reserved0; float half_extent[3]; int32_t reserved1; };
+
+// one axis of a sweep: centre, half extent, normalised direction component, its inverse and sign (step 0: still)
+struct cvxr_axis { float c, h, d, inv; int step; };
+
+// cell k's window on one axis (§3.6 step 2); a still axis has (-inf, +inf) where lo < c < hi and an empty window elsewhere
+__device__ __forceinline__ void cvxr_window(const cvxr_axis& a, int k, int lod, float& enter, float& exit) {
+    const float inf = __builtin_inff();
+    const float lo = (float)(k << lod) - a.h, hi = (float)((k + 1) << lod) + a.h;
+    if (a.step == 0) {
+        const bool in = lo < a.c && a.c < hi;
+        enter = in ? -inf : inf; exit = in ? inf : -inf;
+        return;
+    }
+    const float p = (lo - a.c) * a.inv, q = (hi - a.c) * a.inv;
+    enter = a.step > 0 ? p : q; exit = a.step > 0 ? q : p;
+}
+__device__ __forceinline__ float cvxr_enter(const cvxr_axis& a, int k, int lod) { float e, x; cvxr_window(a, k, lod, e, x); return e; }
+__device__ __forceinline__ float cvxr_exit(const cvxr_axis& a, int k, int lod) { float e, x; cvxr_window(a, k, lod, e, x); return x; }
+
+// First k of [lo, hi] at which `pred` holds, for a predicate that is false then true over [lo, hi); e (a floor) is an estimate.
+template <class P>
+__device__ __forceinline__ int cvxr_first_true(int lo, int hi, float e, P pred) {
+    int k = e >= (float)lo ? (e <= (float)hi ? (int)e : hi) : lo;     // NaN: lo
+    while (k > lo && pred(k - 1)) k--;
+    while (k < hi && !pred(k)) k++;
+    return k;
+}
+
+// The cells [*A, *B) of [lo, hi) whose window has exit > m1, enter < u and enter <= lim (every cell of the still-axis window).
+__device__ __forceinline__ void cvxr_window_cells(const cvxr_axis& a, int lod, float invS, int lo, int hi, float m1, float u, float lim,
+                                                  int* A, int* B) {
+    if (a.step == 0) {
+        *A = cvxr_first_true(lo, hi, floorf((a.c - a.h) * invS), [&](int k) { return a.c < (float)((k + 1) << lod) + a.h; });
+        *B = cvxr_first_true(*A, hi, floorf((a.c + a.h) * invS) + 1.0f, [&](int k) { return !((float)(k << lod) - a.h < a.c); });
+        return;
+    }
+    // in travel order `early` holds for a prefix and `late` for a suffix; the estimates are the box's extent in cells at m1 and tu
+    auto early = [&](int k) { const float e = cvxr_enter(a, k, lod); return e < u && e <= lim; };
+    auto late = [&](int k) { return cvxr_exit(a, k, lod) > m1; };
+    const float tu = u < lim ? u : lim;
+    if (a.step > 0) {
+        *A = cvxr_first_true(lo, hi, floorf((a.c - a.h + m1 * a.d) * invS), late);
+        *B = cvxr_first_true(*A, hi, floorf((a.c + a.h + tu * a.d) * invS) + 1.0f, [&](int k) { return !early(k); });
+    } else {
+        *A = cvxr_first_true(lo, hi, floorf((a.c - a.h + tu * a.d) * invS), early);
+        *B = cvxr_first_true(*A, hi, floorf((a.c + a.h + m1 * a.d) * invS) + 1.0f, [&](int k) { return !late(k); });
+    }
+}
+
+// One box at LOD `lod` (uploaded); use_bounds as in cvxr_cast. out.steps = column headers read.
+__device__ __forceinline__ void cvxr_sweep(const cvxd_world& w, int lod, const cvxd_box& b, bool use_bounds, cvxd_ray_hit& out) {
+    out.hit = -1; out.face = 0; out.cell[0] = out.cell[1] = out.cell[2] = 0; out.distance = 0.0f; out.color = 0; out.steps = 0;
+    const float inf = __builtin_inff();
+    const float maxd = b.max_distance;
+    for (int i = 0; i < 3; i++)
+        if (!cvxr_finite(b.center[i]) || !cvxr_finite(b.direction[i]) || !cvxr_finite(b.half_extent[i]) || !(b.half_extent[i] > 0.0f)) return;
+    if (!(maxd == inf || cvxr_finite(maxd))) return;
+    float d[3], inv[3];
+    int step[3];
+    if (!cvxr_normalise(b.direction, d, inv, step)) return;
+    out.hit = 0;
+    if (!(maxd >= 0.0f)) return;                                     // every candidate has t* >= 0
+    const cvxr_axis ax = {b.center[0], b.half_extent[0], d[0], inv[0], step[0]};
+    const cvxr_axis az = {b.center[2], b.half_extent[2], d[2], inv[2], step[2]};
+    const cvxr_axis ay = {b.center[1], b.half_extent[1], d[1], inv[1], step[1]};
+    const bool xMajor = fabsf(d[0]) >= fabsf(d[2]);
+    const cvxr_axis aM = xMajor ? ax : az, am = xMajor ? az : ax;
+    const int nx = w.dim_x >> lod, ny = w.dim_y >> lod, nz = w.dim_z >> lod;
+    const int nM = xMajor ? nx : nz, nm = xMajor ? nz : nx;
+    const float invS = 1.0f / (float)(1 << lod);
+    const int s = 1 << lod;
+    const cvxd_lod& L = w.lods[lod];
+
+    bool found = false, bOv = false;
+    float bt = inf;                                                  // best t*
+    int bx = 0, by = 0, bz = 0, bFace = 0;
+    uint32_t bColourAt = 0;
+    float lim = maxd;                                                // min(max_distance, best t*): a cell entered later cannot win
+    int steps = 0;
+
+    int MA, MB;
+    cvxr_window_cells(aM, lod, invS, 0, nM, 0.0f, inf, lim, &MA, &MB);
+    const int sM = aM.step < 0 ? -1 : 1, sm = am.step < 0 ? -1 : 1;
+    for (int kM = sM > 0 ? MA : MB - 1; kM >= MA && kM < MB; kM += sM) {
+        float eM, xM;
+        cvxr_window(aM, kM, lod, eM, xM);
+        if (eM > lim) break;
+        if (!(eM < xM)) continue;
+        int mA, mB;
+        cvxr_window_cells(am, lod, invS, 0, nm, eM > 0.0f ? eM : 0.0f, xM, lim, &mA, &mB);
+        for (int km = sm > 0 ? mA : mB - 1; km >= mA && km < mB; km += sm) {
+            float em, xm;
+            cvxr_window(am, km, lod, em, xm);
+            if (em > lim) break;
+            if (!(em < xm)) continue;
+            // column (cx, cz): T and T' of its XZ windows, entry axis x before z on ties
+            const int cx = xMajor ? kM : km, cz = xMajor ? km : kM;
+            const float ex = xMajor ? eM : em, ez = xMajor ? em : eM;
+            const float txz = ez > ex ? ez : ex, uxz = xm < xM ? xm : xM;
+            const int faceXZ = ez > ex ? 4 + (az.step > 0 ? 0 : 1) : (ax.step > 0 ? 0 : 1);
+            const uint4 h = __ldg(L.headers + (size_t)cx * (size_t)L.mul_x + (size_t)cz);
+            steps++;
+            if (!(h.y & 0xffffu)) continue;
+            // y candidates: exit_y > max(T_xz, 0), enter_y < T'_xz, enter_y <= lim, inside the header's [worldMin, worldMax)
+            const int yMin = (int)((h.y >> 16) >> lod), yMax = (int)((h.z + (uint32_t)s - 1u) >> lod);
+            const int ylo = yMin > 0 ? yMin : 0, yhi = yMax < ny ? yMax : ny;
+            if (ylo >= yhi) continue;
+            int A, B;
+            cvxr_window_cells(ay, lod, invS, ylo, yhi, txz > 0.0f ? txz : 0.0f, uxz, lim, &A, &B);
+            if (A >= B) continue;
+            // first solid cell of [lo, hi) in travel order whose own y window is not empty
+            uint32_t colourAt = 0;
+            auto search = [&](int lo, int hi, bool up) {
+                for (;;) {
+                    const int c = lo >= hi ? -1
+                                           : (use_bounds ? cvxr_first_solid_bounds(L, h, lod, lo, hi, up, &colourAt)
+                                                         : cvxr_first_solid_elements(L, h, ny, lo, hi, up, &colourAt));
+                    if (c < 0) return -1;
+                    float e, x;
+                    cvxr_window(ay, c, lod, e, x);
+                    if (e < x) return c;
+                    if (up) lo = c + 1; else hi = c;
+                }
+            };
+            auto tOf = [&](int k) { const float e = cvxr_enter(ay, k, lod); return e > txz ? e : txz; };
+            int f = search(A, B, ay.step >= 0);
+            if (f < 0) continue;
+            float T = tOf(f);
+            if (ay.step < 0) {
+                // T is non-decreasing in travel order, so the cells below f that share its (t*, overlapping) form [g, f]; the lowest
+                // solid one wins
+                const float ts = T > 0.0f ? T : 0.0f;
+                const bool ov = T < 0.0f;
+                const int g = cvxr_first_true(A, f, floorf((ay.c - ay.h + ts * ay.d) * invS), [&](int k) {
+                    const float t = tOf(k);
+                    return (t > 0.0f ? t : 0.0f) == ts && (t < 0.0f) == ov;
+                });
+                if (g < f) { f = search(g, f + 1, true); T = tOf(f); }
+            }
+            const float ts = T > 0.0f ? T : 0.0f;
+            const bool ov = T < 0.0f;
+            const bool better = !found || (ts != bt ? ts < bt
+                                         : ov != bOv ? ov
+                                         : cx != bx ? cx < bx
+                                         : cz != bz ? cz < bz : f < by);
+            if (better) {
+                found = true; bt = ts; bOv = ov; bx = cx; by = f; bz = cz; bColourAt = colourAt;
+                bFace = ov ? 6 : (cvxr_enter(ay, f, lod) > txz ? (ay.step > 0 ? 2 : 3) : faceXZ);
+                lim = bt < maxd ? bt : maxd;
+            }
+        }
+    }
+    out.steps = steps;
+    if (!found) return;
+    out.hit = 1; out.face = bFace; out.distance = bt;
+    out.cell[0] = bx; out.cell[1] = by; out.cell[2] = bz;
+    out.color = __ldg(L.elements + bColourAt);
+}
+
 #ifdef __CUDACC__
 cudaError_t cvxd_launch_raycast(const cvxd_world& world, int lod, const cvxd_ray* rays, cvxd_ray_hit* hits, int n, bool use_bounds,
                                 cudaStream_t stream);
+cudaError_t cvxd_launch_sweep(const cvxd_world& world, int lod, const cvxd_box* boxes, cvxd_ray_hit* hits, int n, bool use_bounds,
+                              cudaStream_t stream);
 #endif

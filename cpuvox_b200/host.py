@@ -189,6 +189,25 @@ def make_rays(origins, directions, max_distance=np.inf) -> np.ndarray:
     return rays
 
 
+# cvx_box as a numpy record (include/cpuvox_b200.h); cvx_sweep returns RAY_HIT_DTYPE records
+BOX_DTYPE = np.dtype([("center", "<f4", 3), ("max_distance", "<f4"), ("direction", "<f4", 3), ("reserved0", "<i4"),
+                      ("half_extent", "<f4", 3), ("reserved1", "<i4")])
+
+
+def make_boxes(centers, half_extents, directions, max_distance=np.inf) -> np.ndarray:
+    """Pack centers (n, 3), half_extents ((n, 3) or (3,)), directions (n, 3) and max_distance (scalar or (n,)) into a cvx_box array."""
+    centers = np.asarray(centers, dtype=np.float32).reshape(-1, 3)
+    directions = np.asarray(directions, dtype=np.float32).reshape(-1, 3)
+    if centers.shape != directions.shape:
+        raise ValueError(f"centers {centers.shape} and directions {directions.shape} differ")
+    boxes = np.zeros(centers.shape[0], dtype=BOX_DTYPE)
+    boxes["center"] = centers
+    boxes["half_extent"] = np.asarray(half_extents, dtype=np.float32)
+    boxes["direction"] = directions
+    boxes["max_distance"] = max_distance
+    return boxes
+
+
 def screen_ray(pose: CameraPose, px: float, py: float, width: int, height: int) -> Tuple[np.ndarray, np.ndarray]:
     """Camera.ScreenPointToRay (cvx_host_screen_ray): pixel (px, py) in Unity screen space (bottom-left origin) of a width x height
     camera; returns (origin on the near plane, normalised direction), float32 (3,) each."""
@@ -371,6 +390,24 @@ class RenderManager:
         """The voxel under screen pixel (px, py) (bottom-left origin) of `pose` at this context's resolution: one RAY_HIT_DTYPE record."""
         o, d = screen_ray(pose, px, py, self.width, self.height)
         return self.raycast(o, d, max_distance, lod)[0]
+
+    # -- swept-box queries (cvx_sweep) ---------------------------------------------------------------
+    def sweep_boxes(self, boxes: np.ndarray, lod: int = 0) -> np.ndarray:
+        """cvx_sweep over a BOX_DTYPE array (host path): returns the RAY_HIT_DTYPE hits."""
+        boxes = np.ascontiguousarray(boxes, dtype=BOX_DTYPE)
+        hits = np.zeros(boxes.shape[0], dtype=RAY_HIT_DTYPE)
+        self._ck(lib.cvx_sweep(self._ctx, _ptr(boxes), boxes.shape[0], lod, _ptr(hits), 0))
+        return hits
+
+    def sweep(self, centers, half_extents, directions, max_distance=np.inf, lod: int = 0) -> np.ndarray:
+        """How far each axis-aligned box moves along its direction before it touches a solid cell of LOD `lod`: centers /
+        directions (n, 3) and half_extents (n, 3) or (3,) in world units, max_distance a scalar or (n,). Returns a RAY_HIT_DTYPE
+        array (hit 1 / 0 / -1 invalid, face of the cell entered or 6 = overlapping at the start, cell, distance, color, steps)."""
+        return self.sweep_boxes(make_boxes(centers, half_extents, directions, max_distance), lod)
+
+    def sweep_device(self, boxes_ptr: int, hits_ptr: int, n: int, lod: int = 0):
+        """cvx_sweep on device arrays (n cvx_box in, n cvx_ray_hit out), ordered on the context's stream; returns at once."""
+        self._ck(lib.cvx_sweep(self._ctx, C.c_void_p(boxes_ptr), n, lod, C.c_void_p(hits_ptr), 1))
 
     # -- outputs ----------------------------------------------------------------------------------
     def read_frame(self, out: Optional[np.ndarray] = None) -> np.ndarray:

@@ -124,6 +124,17 @@ class RayHit(C.Structure):  # cvx_ray_hit, 32 bytes
     ]
 
 
+class Box(C.Structure):  # cvx_box: a swept-box query (no reference analogue), 48 bytes
+    _fields_ = [
+        ("center", C.c_float * 3),
+        ("max_distance", C.c_float),
+        ("direction", C.c_float * 3),
+        ("reserved0", C.c_int32),
+        ("half_extent", C.c_float * 3),
+        ("reserved1", C.c_int32),
+    ]
+
+
 # every symbol include/cpuvox_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _I32, _I64, _U32, _F = C.c_int32, C.c_int64, C.c_uint32, C.c_float
@@ -173,6 +184,7 @@ SYMBOLS = {
     "cvx_ring_consume": (C.c_int, [_P, C.c_int64, _P, C.POINTER(_P)]),
     "cvx_ring_status": (C.c_int, [_P]),
     "cvx_raycast": (C.c_int, [_P, _P, _I32, _I32, _P, _I32]),
+    "cvx_sweep": (C.c_int, [_P, _P, _I32, _I32, _P, _I32]),
     "cvx_debug_ray_setup": (C.c_int, [_P, C.POINTER(FrameSetup), C.POINTER(RayState), _I32]),
     "cvx_debug_ray_timing": (C.c_int, [_P, C.POINTER(FrameSetup), _P, _I32]),
     "cvx_host_quat_euler": (None, [_F, _F, _F, C.POINTER(_F * 4)]),

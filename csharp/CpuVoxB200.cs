@@ -69,6 +69,19 @@ public static unsafe class CpuVoxB200
 		public uint Color; // ColorARGB32
 		public int Steps;
 	}
+
+	// Swept-box queries (cvx_sweep): how far the open box moves before it touches the world. 48 bytes; the result is a RayHit
+	// (Face 6 = the box overlaps the cell at its start, Steps = column headers read).
+	[StructLayout(LayoutKind.Sequential)]
+	public struct Box
+	{
+		public float CenterX, CenterY, CenterZ;
+		public float MaxDistance; // float.PositiveInfinity = unbounded
+		public float DirectionX, DirectionY, DirectionZ; // need not be normalised
+		public int Reserved0;
+		public float HalfExtentX, HalfExtentY, HalfExtentZ; // world units, each > 0
+		public int Reserved1;
+	}
 	[DllImport(LIB)] public static extern int cvx_create(ref Config config, out IntPtr ctx);
 	[DllImport(LIB)] public static extern int cvx_destroy(IntPtr ctx);
 	[DllImport(LIB)] public static extern IntPtr cvx_last_error(IntPtr ctx);
@@ -88,6 +101,7 @@ public static unsafe class CpuVoxB200
 	[DllImport(LIB)] public static extern int cvx_set_option(IntPtr ctx, int option, int value); // 1 lanes per ray, 2 counters, 3 general path, 4 views in flight
 	// onDevice 0: host arrays, returns with the hits; onDevice 1: device pointers, ordered on the context's stream
 	[DllImport(LIB)] public static extern int cvx_raycast(IntPtr ctx, Ray* rays, int n, int lod, RayHit* hits, int onDevice);
+	[DllImport(LIB)] public static extern int cvx_sweep(IntPtr ctx, Box* boxes, int n, int lod, RayHit* hits, int onDevice);
 	// world production on the GPU (VoxelizerHelper + WorldBuilder.ToFinalColumn + World.DownSample as CUDA kernels); positions = n x float3
 	// already in mesh space, colors32 = n x Color32; flips = int[3]. The first returns a builder handle (read its LOD blobs with
 	// cvx_builder_lod, free with cvx_builder_free), the second installs the result as the context's world without a host copy.

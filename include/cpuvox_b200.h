@@ -265,6 +265,31 @@ typedef struct cvx_ray_hit {
  * n == 0 does nothing. CVX_OPT_GENERAL_PATH 1 makes it read runs from the element area (same results). */
 int cvx_raycast(cvx_ctx* ctx, const cvx_ray* rays, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device);
 
+/* Swept boxes: how far can an axis-aligned box move before it touches the world, and which face stops it? Camera collision,
+ * character controllers, projectiles with a radius, free-space checks for a spawn position. The open box of half extents
+ * `half_extent` (world units, each > 0) centred on `center` moves along `direction` (need not be normalised) up to `max_distance`
+ * (world units along the normalised direction; +inf allowed). The result reuses cvx_ray_hit; the exact definition, which the device
+ * kernel follows bit for bit in IEEE fp32, is DESIGN.md §3.6:
+ *   hit       1 = the box touches a solid cell of LOD j within max_distance, 0 = it does not, -1 = invalid box (a NaN / infinite
+ *             input other than max_distance = +inf, a half extent <= 0, or a zero-length direction)
+ *   distance  how far the box moves before it overlaps the cell (touching or grazing a face is not contact, so a box resting on a
+ *             floor slides along it); 0 when it overlaps the cell where it starts
+ *   face      outward normal of the cell face the box enters through, numbered as for cvx_raycast; 6 = the box overlaps the cell
+ *             already at its start
+ *   cell      the first such cell, ties broken by lowest x, then z, then y; color its ColorARGB32
+ *   steps     column headers the query read (a cost figure, not part of the definition)
+ * A miss or an invalid box has every field but `steps` zero. Arguments, errors, host and device arrays, stream ordering and scratch
+ * behave as for cvx_raycast (the two share the scratch). The cost per box grows with its XZ footprint in cells and its travel. */
+typedef struct cvx_box {
+    float center[3];
+    float max_distance;
+    float direction[3];
+    int32_t reserved0;
+    float half_extent[3];
+    int32_t reserved1;
+} cvx_box; /* 48 bytes */
+int cvx_sweep(cvx_ctx* ctx, const cvx_box* boxes, int32_t n, int32_t lod, cvx_ray_hit* out, int32_t on_device);
+
 /* Debug: dump the per-ray state after RaySetupJob/DDASetupJob/TraceToFirstColumnJob
  * (DrawSegmentRayJob.cs:12-144) for every flat ray index; 18 x 4 bytes per ray, see cvx_ray_state. */
 typedef struct cvx_ray_state {

@@ -14,7 +14,8 @@ namespace {
 
 struct Ray { float origin[3]; float max_distance; float direction[3]; int32_t reserved; };
 struct Hit { int32_t hit; int32_t face; int32_t cell[3]; float distance; uint32_t color; int32_t steps; };
-static_assert(sizeof(Ray) == 32 && sizeof(Hit) == 32, "layouts");
+struct Box { float center[3]; float max_distance; float direction[3]; int32_t reserved0; float half_extent[3]; int32_t reserved1; };
+static_assert(sizeof(Ray) == 32 && sizeof(Hit) == 32 && sizeof(Box) == 48, "layouts");
 
 struct Lod { const uint8_t* blob; int64_t bytes; int32_t column_count; };
 
@@ -61,21 +62,13 @@ float tmax_of(int cell, int step, int lod, float o, float inv) {
     return ((float)((cell + (step > 0 ? 1 : 0)) << lod) - o) * inv;
 }
 
-void cast(const World& w, int lod, const Ray& r, Hit& out) {
-    memset(&out, 0, sizeof out);
-    out.hit = -1;
-    // 1. normalise
-    for (int i = 0; i < 3; i++)
-        if (!finite(r.origin[i]) || !finite(r.direction[i])) return;
-    if (std::isnan(r.max_distance) || r.max_distance == -INFINITY) return;
-    const float dx = r.direction[0], dy = r.direction[1], dz = r.direction[2];
-    const float len2 = dx * dx + dy * dy + dz * dz;
-    if (!(len2 > 0.0f) || !finite(len2)) return;
+// step 1 of §3.5 and §3.6: false when the squared length is 0 or not finite
+bool normalise(const float dir[3], float d[3], float inv[3], int step[3]) {
+    const float len2 = dir[0] * dir[0] + dir[1] * dir[1] + dir[2] * dir[2];
+    if (!(len2 > 0.0f) || !finite(len2)) return false;
     const float invLen = 1.0f / sqrtf(len2);
-    float d[3], inv[3];
-    int step[3];
     for (int i = 0; i < 3; i++) {
-        d[i] = r.direction[i] * invLen;
+        d[i] = dir[i] * invLen;
         inv[i] = 0.0f;
         step[i] = 0;
         if (d[i] != 0.0f) {
@@ -84,6 +77,19 @@ void cast(const World& w, int lod, const Ray& r, Hit& out) {
             else d[i] = 0.0f;
         }
     }
+    return true;
+}
+
+void cast(const World& w, int lod, const Ray& r, Hit& out) {
+    memset(&out, 0, sizeof out);
+    out.hit = -1;
+    // 1. normalise
+    for (int i = 0; i < 3; i++)
+        if (!finite(r.origin[i]) || !finite(r.direction[i])) return;
+    if (std::isnan(r.max_distance) || r.max_distance == -INFINITY) return;
+    float d[3], inv[3];
+    int step[3];
+    if (!normalise(r.direction, d, inv, step)) return;
     out.hit = 0;
     const float* o = r.origin;
     const float maxd = r.max_distance;
@@ -141,6 +147,105 @@ void cast(const World& w, int lod, const Ray& r, Hit& out) {
     }
 }
 
+// cvx_sweep (DESIGN.md §3.6) evaluated cell by cell over the swept box's bounding box: on each axis the cells whose own window
+// meets [0, max_distance] (a cell outside that set cannot be a candidate: T >= enter_i, T' <= exit_i). steps stays 0.
+struct Window { int k; float enter, exit; };
+
+void sweep(const World& w, int lod, const Box& b, Hit& out) {
+    memset(&out, 0, sizeof out);
+    out.hit = -1;
+    // 1. invalid inputs, normalise
+    for (int i = 0; i < 3; i++)
+        if (!finite(b.center[i]) || !finite(b.direction[i]) || !finite(b.half_extent[i]) || !(b.half_extent[i] > 0.0f)) return;
+    const float maxd = b.max_distance;
+    if (std::isnan(maxd) || maxd == -INFINITY) return;
+    float d[3], inv[3];
+    int step[3];
+    if (!normalise(b.direction, d, inv, step)) return;
+    out.hit = 0;
+    const int n[3] = {w.dims[0] >> lod, w.dims[1] >> lod, w.dims[2] >> lod};
+    // 2. per-axis windows
+    std::vector<Window> win[3];
+    for (int i = 0; i < 3; i++) {
+        const float c = b.center[i], h = b.half_extent[i];
+        for (int k = 0; k < n[i]; k++) {
+            const float lo = (float)(k << lod) - h, hi = (float)((k + 1) << lod) + h;
+            float enter, exit;
+            if (step[i] == 0) {
+                if (!(lo < c && c < hi)) continue;
+                enter = -INFINITY;
+                exit = INFINITY;
+            } else {
+                const float a = (lo - c) * inv[i], bb = (hi - c) * inv[i];
+                enter = step[i] > 0 ? a : bb;
+                exit = step[i] > 0 ? bb : a;
+            }
+            if (enter < exit && exit > 0.0f && enter <= maxd) win[i].push_back(Window{k, enter, exit});
+        }
+    }
+    // 3. candidates, 4. the smallest key (t*, overlapping first, cx, cz, cy)
+    bool found = false, bestOv = false;
+    float bestT = 0.0f;
+    int best[3] = {0, 0, 0}, bestFace = 0;
+    uint32_t bestColour = 0;
+    for (const Window& X : win[0])
+        for (const Window& Z : win[2]) {
+            // the XZ part alone already rules the column out (max and min only grow and shrink with the y window)
+            const float txz = Z.enter > X.enter ? Z.enter : X.enter, uxz = Z.exit < X.exit ? Z.exit : X.exit;
+            if (!(txz < uxz) || !(txz <= maxd)) continue;
+            for (const Window& Y : win[1]) {
+                float T = X.enter;
+                int axis = 0;
+                if (Z.enter > T) { T = Z.enter; axis = 2; }
+                if (Y.enter > T) { T = Y.enter; axis = 1; }
+                float Tp = X.exit;
+                if (Z.exit < Tp) Tp = Z.exit;
+                if (Y.exit < Tp) Tp = Y.exit;
+                const float ts = T > 0.0f ? T : 0.0f;
+                if (!(T < Tp && Tp > 0.0f && ts <= maxd && finite(ts))) continue;
+                const bool ov = T < 0.0f;
+                const int cell[3] = {X.k, Y.k, Z.k};
+                bool better = !found;
+                if (found) {
+                    if (ts != bestT) better = ts < bestT;
+                    else if (ov != bestOv) better = ov;
+                    else if (cell[0] != best[0]) better = cell[0] < best[0];
+                    else if (cell[2] != best[2]) better = cell[2] < best[2];
+                    else better = cell[1] < best[1];
+                }
+                if (!better) continue;
+                uint32_t colour = 0;
+                if (!solid(w, lod, cell[0], cell[1], cell[2], &colour)) continue;
+                found = true; bestT = ts; bestOv = ov; bestColour = colour;
+                best[0] = cell[0]; best[1] = cell[1]; best[2] = cell[2];
+                bestFace = ov ? 6 : 2 * axis + (step[axis] > 0 ? 0 : 1);
+            }
+        }
+    if (!found) return;
+    out.hit = 1; out.face = bestFace; out.distance = bestT; out.color = bestColour;
+    out.cell[0] = best[0]; out.cell[1] = best[1]; out.cell[2] = best[2];
+}
+
+// body(i) for i in [0, n) on `threads` host threads (<= 0: all hardware threads), `chunk` queries at a time
+template <class F>
+void parallel(int n, int threads, int chunk, F body) {
+    if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
+    if (threads < 1) threads = 1;
+    std::atomic<int> next{0};
+    auto worker = [&]() {
+        for (;;) {
+            const int b = next.fetch_add(chunk);
+            if (b >= n) break;
+            const int e = b + chunk < n ? b + chunk : n;
+            for (int i = b; i < e; i++) body(i);
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 1; t < threads; t++) pool.emplace_back(worker);
+    worker();
+    for (auto& t : pool) t.join();
+}
+
 } // namespace
 
 extern "C" {
@@ -168,22 +273,17 @@ int rco_raycast(const void* world, int32_t lod, const void* rays, int32_t n, voi
     if (!w || lod < 0 || lod >= 6 || !w->lods[lod].blob || n < 0) return -1;
     const Ray* in = (const Ray*)rays;
     Hit* out = (Hit*)hits;
-    if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
-    if (threads < 1) threads = 1;
-    const int chunk = 1024;
-    std::atomic<int> next{0};
-    auto worker = [&]() {
-        for (;;) {
-            const int b = next.fetch_add(chunk);
-            if (b >= n) break;
-            const int e = b + chunk < n ? b + chunk : n;
-            for (int i = b; i < e; i++) cast(*w, lod, in[i], out[i]);
-        }
-    };
-    std::vector<std::thread> pool;
-    for (int t = 1; t < threads; t++) pool.emplace_back(worker);
-    worker();
-    for (auto& t : pool) t.join();
+    parallel(n, threads, 1024, [&](int i) { cast(*w, lod, in[i], out[i]); });
+    return 0;
+}
+
+// n boxes at LOD lod on `threads` host threads (<= 0: all hardware threads)
+int rco_sweep(const void* world, int32_t lod, const void* boxes, int32_t n, void* hits, int32_t threads) {
+    const World* w = (const World*)world;
+    if (!w || lod < 0 || lod >= 6 || !w->lods[lod].blob || n < 0) return -1;
+    const Box* in = (const Box*)boxes;
+    Hit* out = (Hit*)hits;
+    parallel(n, threads, 64, [&](int i) { sweep(*w, lod, in[i], out[i]); });
     return 0;
 }
 

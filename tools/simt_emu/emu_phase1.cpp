@@ -155,4 +155,24 @@ int emu_raycast(const emu_world* w, int lod, const cvxd_ray* rays, int n, cvxd_r
     return 0;
 }
 
+// cvx_sweep's traversal (raycast.h) for boxes [0, n) at LOD lod, one call per box as one device thread runs it; general as above.
+int emu_sweep(const emu_world* w, int lod, const cvxd_box* boxes, int n, cvxd_ray_hit* hits, int general, int threads) {
+    if (lod < 0 || lod >= w->w.lod_count || n < 0) return -1;
+    const bool bounds = w->tables[lod].regular && !general;
+    std::atomic<int> next{0};
+    if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
+    auto worker = [&]() {
+        for (;;) {
+            const int b = next.fetch_add(256);
+            if (b >= n) break;
+            for (int i = b; i < n && i < b + 256; i++) cvxr_sweep(w->w, lod, boxes[i], bounds, hits[i]);
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int t = 1; t < threads; t++) pool.emplace_back(worker);
+    worker();
+    for (auto& t : pool) t.join();
+    return 0;
+}
+
 } // extern "C"
